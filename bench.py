@@ -5,10 +5,10 @@ Workload (config.workload): BASELINE config 4, "P1 tet Poisson 64M tets" -- the 
 quoted on: Kuhn cube n=220, 63,888,000 C3D4 tets, 10,793,861 nodes, CSR nnz 160,738,381, fp64.  It fits one B200.
 A step = one CG iteration of the reference's projected CG (solver.py:144-229) on the assembled CSR operator.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--n 220] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--n 220] [--impl reference] [--dump-outputs DIR]
 
-Prints ONE JSON line (rank 0).  `value` = CG iterations/s with everything resident in HBM (device events around the
-graph-captured loop), `e2e` = the same through the public solver API with the load vector in pinned host memory and the
+Prints ONE JSON line (rank 0).  `value` = CG iterations/s with everything resident in HBM (device events around one
+graph-captured loop of exactly K iterations), `e2e` = the same through the public solver API with the load vector in pinned host memory and the
 solution read back to the host inside the timed region of every call (median of repeated calls; the first call of the
 process is reported as `first_call_ms`).  `roofline` is for the dominant kernel (the CSR SpMV).
 `assembly` reports the second half of the metric (assembled elems/s, fused coords->CSR values) with its own roofline.
@@ -16,8 +16,12 @@ process is reported as `first_call_ms`).  `roofline` is for the dominant kernel 
 `--impl reference` times the UNMODIFIED reference (baseline/_ref/solver, installed by __graft_entry__.build(); run by
 baseline/ref_arm.py in a subprocess, torch CPU on all host threads) on a bounded sample of the same workload; the C
 restatement under oracle/ is reported beside it as a labelled second baseline (`cpu_baseline.port`).
+`--dump-outputs DIR` (1 GPU) writes what the timed paths returned in their last step as DIR/<name>.npy (float64): the CG
+solution and final r.r, the solution of the last e2e call and the assembled CSR values.  Inputs are seeded, so two builds
+run with the same arguments can be compared output for output.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -65,6 +69,7 @@ class ClockSampler:
         try:
             self.p = subprocess.Popen(["nvidia-smi", f"--id={index}", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "20"],
                                       stdout=self.f, stderr=subprocess.DEVNULL)
+            atexit.register(self.stop)     # an exception before stop() must not leave nvidia-smi running
         except OSError:
             self.p = None
 
@@ -77,6 +82,7 @@ class ClockSampler:
             self.p.wait(timeout=5)
         except Exception:
             self.p.kill()
+        self.p = None
         self.f.flush()
         rows = [r.split(",") for r in open(self.f.name).read().strip().splitlines() if r.count(",") >= 9]
         os.unlink(self.f.name)
@@ -98,6 +104,29 @@ class ClockSampler:
         out["reasons"] = [n for k, n in enumerate(names) if any("Active" in r[5 + k] and "Not" not in r[5 + k] for r in rows)]
         out["samples"] = len(rows)
         return out
+
+
+# ------------------------------------------------------------------------------------------------ --dump-outputs
+DUMP_SAMPLE = 1 << 21      # entries kept of a larger output (16 MB in float64), so that a dump stays well under 64 MB
+
+
+def dump_sample(t):
+    """`t` flattened to a float64 host array; an output of more than DUMP_SAMPLE entries is cut to a fixed sample of them
+    (numpy seed 0, sorted indices), which depends only on the output's size."""
+    import numpy as np
+    import torch
+    t = t.reshape(-1)
+    if t.numel() > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_SAMPLE, replace=False))
+        t = t[torch.from_numpy(idx).to(t.device)]
+    return t.to("cpu", torch.float64).numpy()
+
+
+def write_outputs(path, outputs):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------ CPU side (oracle)
@@ -208,6 +237,7 @@ def config2(dev, hbm, n=69, iters=100):
 
 # ------------------------------------------------------------------------------------------------ GPU arm
 def run_gpu(args):
+    import numpy as np
     import torch
     import torch.distributed as dist
     import element as el
@@ -220,9 +250,11 @@ def run_gpu(args):
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device(f"cuda:{local}"))
     torch.cuda.set_device(local)
+    torch.manual_seed(0)
     dev = torch.device(f"cuda:{local}")
     n = args.n
     K, W = args.steps, max(args.warmup, 3)
+    outputs = {}            # --dump-outputs: name -> host array
 
     if world > 1:
         from femb200 import dist_cg
@@ -260,6 +292,8 @@ def run_gpu(args):
     a1.record()
     torch.cuda.synchronize()
     ms_asm = a0.elapsed_time(a1) / reps_a
+    if args.dump_outputs:
+        outputs["assembly_csr_values"] = dump_sample(vals)
     bytes_asm = M * 4 * 8 + N * 24 + nnz * 8          # SURVEY 8d: conn as the API receives it (int64) + coords + values
     # drop-in element matrices (compute_K_matrix path), Poisson 4x4
     Ke = el.compute_c3d4_poisson_K_matrix(coords, tets, device=dev, dtype=torch.float64)
@@ -317,14 +351,9 @@ def run_gpu(args):
     ms_call = c0.elapsed_time(c1)
     ms_loop = info["loop_ms"]
     assert info["iterations"] == K, info
-    # a K-step loop of a few milliseconds is at the mercy of one clock ramp: the same EXACTLY-K-step solve is repeated until
-    # >= 50 ms have been timed in total and the median is reported (`timed_repeats` in the line)
-    loops = [ms_loop]
-    while sum(loops) < 50.0 and len(loops) < 25:
-        _, info_r = ops.cg_solve(crow, col, vals, F, mask=mask, tol=0.0, max_iter=K, check_every=min(K, 50))
-        loops.append(info_r["loop_ms"])
-    loops.sort()
-    ms_loop = loops[len(loops) // 2]
+    if args.dump_outputs:
+        outputs["cg_u"] = dump_sample(u)
+        outputs["cg_rs"] = np.array([info["rs"]], dtype=np.float64)
     bytes_iter = bytes_spmv + 9 * N * 8                 # SURVEY 8d
 
     # ---- e2e: public solver API, load vector from pinned host memory, solution read back to the host
@@ -351,6 +380,8 @@ def run_gpu(args):
         e2e_ms.append(ms_c)
     e2e_ms.sort()
     ms_e2e = e2e_ms[len(e2e_ms) // 2]
+    if args.dump_outputs:
+        outputs["e2e_u"] = dump_sample(u_host)
     t_soak = time.perf_counter()           # untimed: keep the same loop running until the sampler has >= 0.5 s under load
     while time.perf_counter() - t_soak < 0.5:
         ops.cg_solve(crow, col, vals, F, mask=mask, tol=0.0, max_iter=200, check_every=50)
@@ -398,7 +429,7 @@ def run_gpu(args):
                 "calls": len(e2e_ms), "first_call_ms": round(ms_e2e_first, 3), "ms_per_call": round(ms_e2e, 3),
                 "note": f"one solver-API call of {K} iterations: F pinned host -> device, CG, u -> pinned host; bytes are per call / K; "
                         "median over `calls` identical calls after one untimed-in-the-median first call"},
-        "gpu_launches": (3 if os.environ.get("FEMB_CG_CLASSIC") else 2) * K + 4, "timed_repeats": len(loops),
+        "gpu_launches": (3 if os.environ.get("FEMB_CG_CLASSIC") else 2) * K + 4,
         "roofline": {"kernel": "spmv_tma_kernel<1,false> (TMA-pipelined CSR SpMV; its fused twin is CG step k1)", "bound": "hbm",
                      "achieved": round(bytes_spmv / (ms_spmv * 1e-3) / 1e9, 1), "peak": hbm, "unit": "GB/s",
                      "frac": round(bytes_spmv / (ms_spmv * 1e-3) / 1e9 / hbm, 4), "traffic": ncu_traffic(n, "spmv_tma_kernel"), "peak_source": peak_src,
@@ -431,6 +462,8 @@ def run_gpu(args):
     if not args.no_cpu:
         out["cpu_baseline"] = cpu_baseline_leg(args, nnz)
     print(json.dumps(out), flush=True)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
 
 
 def cpu_baseline_leg(args, nnz):
@@ -557,7 +590,10 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-topo", action="store_true", help="skip the face-connectivity timing on the headline mesh")
     ap.add_argument("--no-c2", action="store_true", help="skip the secondary BASELINE config 2 (P2 elasticity) measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the timed paths' last step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "femb200" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs is supported on the single-GPU femb200 arm")
     if args.impl == "reference":
         run_reference(args)
     else:
