@@ -79,6 +79,10 @@ SIGNATURES = {
     "femb_mv_gram": [c_i64, c_i32, c_vp, c_i64, c_i32, c_vp, c_i64, c_vp, C.POINTER(c_f64), c_vp],
     "femb_mv_update": [c_i64, c_i32, c_vp, c_i64, c_i32, C.POINTER(c_f64), c_f64, c_vp, c_i64, c_vp],
     "femb_mv_scale_mask": [c_i64, c_i32, c_vp, c_i64, c_vp, c_vp, c_vp],
+    "femb_spmm_bsr3": [c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_i64, c_vp, c_vp, c_i64, c_vp],
+    "femb_mb_gram": [c_i64, c_i32, c_vp, c_i64, c_i32, c_vp, c_i64, c_vp, c_vp],
+    "femb_mb_combine": [c_i64, c_i32, c_vp, c_i64, c_i32, C.POINTER(c_f64), c_f64, c_vp, c_i64, c_vp],
+    "femb_lobpcg_residual": [c_i64, c_i32, c_vp, c_i64, c_vp, c_vp, c_i64, C.POINTER(c_f64), c_vp, c_i32, c_vp, c_vp, c_i64, c_vp, c_vp],
     "femb_csr_jacobi": [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp],
     "femb_graph_from_pairs": [c_vp, c_i64, c_i32, c_i64, c_vp, c_vp, c_vp],
     "femb_subdomain_forces": [c_vp, c_i32, c_i64, c_i32, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp],

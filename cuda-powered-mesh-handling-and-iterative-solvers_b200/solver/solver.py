@@ -472,7 +472,8 @@ def vectorized_modal_solver(K_local, M_local, elements, rbe2_node_ids, num_nodes
     The n_dof-long work runs on the device in fp64: K is assembled once (3x3 block-CSR) and applied column by column, the lumped
     mass comes from one pass over the incidence lists, and norms / projections / X^T K X / X Z are three tall-skinny kernels
     (femb_mv_*); only the k x k problems are solved on the host.  The reference
-    draws its start subspace from an unseeded torch.randn; pass `X0` [3*num_nodes, num_eigs] (additive) for a reproducible run."""
+    draws its start subspace from an unseeded torch.randn; pass `X0` [3*num_nodes, num_eigs] (additive) for a reproducible run.
+    For the lowest natural frequencies and mode shapes use `lowest_modes`."""
     dev = _ops.cuda_device(device)
     if not 1 <= num_eigs <= 8:
         raise ValueError("num_eigs must be between 1 and 8")
@@ -515,6 +516,44 @@ def vectorized_modal_solver(K_local, M_local, elements, rbe2_node_ids, num_nodes
     lam, Z = gevp(X)
     X.update_into(torch.from_numpy(Z.astype("float64")), X)
     return torch.from_numpy(lam.copy()).to(device=dev, dtype=dtype), X.columns().to(dtype)
+
+
+def lowest_modes(K_local, M_local, elements, fixed, num_nodes, num_eigs=6, tol=1e-8, max_iter=2000, X0=None, device="cuda:0",
+                 dtype=torch.float64, return_info=False, verbose=True):
+    """Lowest eigenpairs of K x = lam M x for 3-dof solid meshes (not in the reference): LOBPCG with a Jacobi preconditioner
+    (femb200/modes.py).  K_local, M_local: element matrices [M, 3 nen, 3 nen] of any solid type (a lumped mass is a diagonal
+    M_local); both are assembled on one plan into 3x3 block-CSR with one block pattern.  `fixed`: node ids or a bool node mask, all
+    three dofs clamped; the result is the eigenpairs of the reduced pencil (K_ff, M_ff) with zeros on the fixed dofs (with `fixed`
+    empty the six rigid-body modes come out at lam = 0).  1 <= num_eigs <= 12.
+
+    A pair has converged when |K x - lam M x| / ((|K|_1 + |lam| |M|_1) |x|) <= tol; the solve stops when the first num_eigs have,
+    or after max_iter iterations with status "maxiter" (it does not raise).  X0 [3*num_nodes, num_eigs] is optional; the rest of
+    the start block comes from a fixed-seed generator, so a repeated call returns bit-identical results.
+    Returns (lam [num_eigs] ascending, modes [3*num_nodes, num_eigs] M-orthonormal), cast to `dtype`; with return_info also a dict
+    with iterations, status, residuals, restarts (iterations that dropped the P block), freq_hz = sqrt(max(lam, 0)) / 2 pi, loop_ms."""
+    from femb200 import modes
+    dev = _ops.cuda_device(device)
+    if not 1 <= num_eigs <= 12:
+        raise ValueError("num_eigs must be between 1 and 12")
+    n = 3 * num_nodes
+    if X0 is not None:
+        X0 = torch.as_tensor(X0).to(torch.float64).cpu().numpy()
+        if X0.shape != (n, num_eigs):
+            raise ValueError(f"X0 must be [{n}, {num_eigs}]")
+    plan = _ops.cached_plan(elements, num_nodes, dev)
+    brow, bcol = plan.pattern(1)
+    K = _ops.Bsr3.from_csr_values(brow, bcol, plan.assemble(K_local, 3))
+    M = _ops.Bsr3.from_csr_values(brow, bcol, plan.assemble(M_local, 3))
+    be = modes.DeviceBackend(K, M, _dof_mask(num_nodes, 3, fixed, dev))
+    lam, S, info = modes.lobpcg(be, num_eigs, tol=tol, max_iter=max_iter, X0=X0)
+    if verbose:
+        if info["status"] == "converged":
+            print(f"LOBPCG converged after {info['iterations']} iterations ({info['restarts']} restarts).")
+        else:
+            print(f"LOBPCG did not converge within {max_iter} iterations; max residual {info['residuals'].max():.3e}.")
+    lam = torch.from_numpy(lam).to(device=dev, dtype=dtype)
+    modes_out = S[:, :num_eigs].contiguous().to(dtype)
+    return (lam, modes_out, info) if return_info else (lam, modes_out)
 
 
 def static_structure_solver(coords, force, fixed, c3d4=None, c3d6=None, c3d8=None, s3=None, s4=None, material=None, u_init=None,

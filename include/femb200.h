@@ -302,6 +302,24 @@ int femb_mv_update(int64_t n, int ki, const double* X, int64_t ldx, int kj, cons
                    femb_stream stream);
 int femb_mv_scale_mask(int64_t n, int k, double* X, int64_t ldx, const double* scale, const uint8_t* mask, femb_stream stream);
 
+/* Block kernels of the LOBPCG modal solver (lowest_modes, not in the reference).  Multivectors are ROW-MAJOR and node-interleaved:
+ * value (dof r, column j) at X[r*ld + j], ld >= the columns used.  Sums are deterministic (fixed-order two-stage reductions, no
+ * atomics); outputs must not overlap inputs (views of one buffer with the same ld and disjoint columns are allowed).
+ *   femb_spmm_bsr3: YK = K X and, when mval != NULL, YM = M X in the same pass; K and M share brow/bcol (3x3 blocks as in
+ *     femb_spmv_bsr3), 1 <= m <= 16 columns; mask (NULL: none) zeroes x and y on dofs with mask == 0.
+ *   femb_mb_gram: G[i*kb+j] = sum_r A[r*lda+i] B[r*ldb+j], 1 <= ka, kb <= 48; G is a device array.
+ *   femb_mb_combine: Y[:, :mc] = beta Y[:, :mc] + X[:, :k] C_host (C_host [k, mc] row-major), 1 <= k <= 48, 1 <= mc <= 16.
+ *   femb_lobpcg_residual: r_j = KX_j - lam_host[j] MX_j for j < m (KX, MX share ldk); norms[j] = |r_j|^2, norms[m+j] = |X_j|^2;
+ *     W[:, a] = dinv * r_{active[a]} for a < na (active: device int32 list). */
+int femb_spmm_bsr3(int64_t nb, int64_t nnzb, const int32_t* brow, const int32_t* bcol, const double* kval, const double* mval,
+                   const uint8_t* mask, int m, const double* X, int64_t ldx, double* YK, double* YM, int64_t ldy, femb_stream stream);
+int femb_mb_gram(int64_t n, int ka, const double* A, int64_t lda, int kb, const double* B, int64_t ldb, double* G, femb_stream stream);
+int femb_mb_combine(int64_t n, int k, const double* X, int64_t ldx, int mc, const double* C_host, double beta, double* Y, int64_t ldy,
+                    femb_stream stream);
+int femb_lobpcg_residual(int64_t n, int m, const double* X, int64_t ldx, const double* KX, const double* MX, int64_t ldk,
+                         const double* lam_host, const double* dinv, int na, const int32_t* active, double* W, int64_t ldw,
+                         double* norms, femb_stream stream);
+
 /* Jacobi diagonal of a CSR matrix: minv[i] = mask[i] ? 1/A_ii : 0 (the documented replacement for the
  * reference's broken compute_diagonal_preconditioner solver.py:814-833) */
 int femb_csr_jacobi(int64_t n, const int32_t* crow, const int32_t* col, const double* val, const uint8_t* mask,
