@@ -85,6 +85,10 @@ struct SolveCtx {
   // re-launches the instantiated graph instead of capturing + instantiating again (~1 ms per solve: most of a small solve)
   void* dev_scratch = nullptr;
   size_t dev_scratch_bytes = 0;
+  // 16-bit delta-encoded column index of the merged CG loop (krylov.cu, idx16_encode_kernel): failed-tile counter, one flag
+  // byte per 128-row tile, then col16 (2 bytes per nonzero), re-encoded by every solve that uses it
+  void* idx16 = nullptr;
+  size_t idx16_bytes = 0;
   cudaGraphExec_t graph_exec = nullptr;
   unsigned char graph_key[512];
   size_t graph_key_bytes = 0;

@@ -1110,6 +1110,7 @@ extern "C" int femb_dist_cg_solve(int rank, int nranks, int64_t n_owned, int64_t
     result_host->status = hfin->status;
     result_host->rs = hfin->rs_new;
     result_host->loop_ms = pms;
+    result_host->index_bytes = 4;
     return FEMB_OK;
   }
   if (bptr != nullptr && nnbr > 0 && n_interior > 0 && !getenv("FEMB_DIST_SEPARATE_PUSH")) dist_push_kernel<<<gp, 256, 0, s>>>(pe, send_idx, st);
@@ -1192,6 +1193,7 @@ extern "C" int femb_dist_cg_solve(int rank, int nranks, int64_t n_owned, int64_t
   result_host->status = fin->stop ? fin->status : 2;
   result_host->rs = fin->rs_new;
   result_host->loop_ms = ms;
+  result_host->index_bytes = 4;
   if (trace && fin->it > 20) {  // average phase times over iterations 10..min(it,TRACE_ITERS)-1 (microseconds)
     static long long h[TRACE_ITERS * 12];
     cudaMemcpy(h, trace, sizeof(h), cudaMemcpyDeviceToHost);

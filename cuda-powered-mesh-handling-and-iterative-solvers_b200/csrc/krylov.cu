@@ -183,6 +183,54 @@ __global__ void __launch_bounds__(TMA_THREADS) spmv_tma_kernel(long long n, long
   }
 }
 
+// same with the 16-bit delta-encoded column stream (LR = 1, merged CG loop): col16 / tile_ok from idx16_encode_kernel
+template <bool FUSED>
+__global__ void __launch_bounds__(TMA_THREADS) spmv_tma16_kernel(long long n, long long nnz, const int* __restrict__ crow, const int* __restrict__ col,
+                                                                 const double* __restrict__ val, const double* __restrict__ x,
+                                                                 double* __restrict__ y, const unsigned char* __restrict__ mask,
+                                                                 double* __restrict__ partial, CGState* __restrict__ st, double eps, int guards,
+                                                                 const double* __restrict__ rvec, double tol, long long pin,
+                                                                 const double* __restrict__ wvec, const unsigned short* __restrict__ col16,
+                                                                 const unsigned char* __restrict__ tile_ok) {
+  pdl_launch_dependents();
+  double extra[2] = {0.0, 0.0};
+  const double dot = spmv_tma16_rows<TMA16_STAGES, TMA16_CAP>(n, nnz, crow, col, col16, tile_ok, val, x, y, mask, (guards & 2) != 0, FUSED, rvec,
+                                                             rvec ? extra : nullptr, st ? &st->stop : nullptr, pin, wvec);
+  if (st && st->stop) return;
+  if (FUSED) {
+    if (rvec) cg_k1_epilogue3_n<TMA_THREADS>(dot, extra[0], extra[1], partial, st, eps, guards & 1, tol);
+    else cg_k1_epilogue_n<TMA_THREADS>(dot, partial, st, eps, guards & 1);
+  }
+}
+
+// 16-bit column index: col16[a] = row - col[a] for the first entry a of a row, col16[j] = col[j] - col[j-1] after it.  One CTA
+// per 128-row tile (the tile of spmv_tma16_kernel); tile_ok[t] = 1 when every row of the tile encodes losslessly (first column
+// 0..65535 below the row, strictly increasing columns with gaps <= 65535), and *bad counts the tiles that do not.
+__global__ void __launch_bounds__(TMA_THREADS) idx16_encode_kernel(long long n, const int* __restrict__ crow, const int* __restrict__ col,
+                                                                   unsigned short* __restrict__ col16, unsigned char* __restrict__ tile_ok,
+                                                                   int* __restrict__ bad) {
+  const long long ntiles = (n + TMA_THREADS - 1) / TMA_THREADS;
+  for (long long t = blockIdx.x; t < ntiles; t += gridDim.x) {
+    const long long r = t * TMA_THREADS + threadIdx.x;
+    bool ok = true;
+    if (r < n) {
+      const int a = __ldg(crow + r), b = __ldg(crow + r + 1);
+      long long prev = r;
+      for (int j = a; j < b; ++j) {
+        const long long c = __ldg(col + j), d = j == a ? prev - c : c - prev;
+        ok = ok && d >= (j == a ? 0 : 1) && d <= 65535;
+        col16[j] = (unsigned short)d;
+        prev = c;
+      }
+    }
+    ok = __syncthreads_and(ok);
+    if (threadIdx.x == 0) {
+      tile_ok[t] = ok ? 1 : 0;
+      if (!ok) atomicAdd(bad, 1);
+    }
+  }
+}
+
 // block-CSR (3x3) variant for 3-dof operators: n = 3 nb scalar rows, crow/col are the node-level pattern, val the blocks
 template <int LR, bool FUSED>
 __global__ void __launch_bounds__(TMA_THREADS) spmv_bsr3_tma_kernel(long long nb, long long nnzb, const int* __restrict__ brow,
@@ -487,6 +535,9 @@ static int pick_lanes(long long n, long long nnz, int block = 1) {
 static thread_local long long nnz_hint = 0;  // set by the callers right before launch_spmv (the TMA kernel clamps its copies to nnz)
 static thread_local bool pdl_hint = false;   // launch the next TMA SpMV with the programmatic-serialization attribute (graph loop only)
 static thread_local long long pin_hint = 0;  // leading nonzeros staged evict_last (spmv_pin_entries), 0 outside solves
+// set: lanes == 101 launches spmv_tma16_kernel on this encoded index (cg_solve_impl only)
+static thread_local const unsigned short* col16_hint = nullptr;
+static thread_local const unsigned char* tile_ok_hint = nullptr;
 
 template <bool FUSED>
 static void launch_spmv(int lanes, int grid, cudaStream_t s, long long n, const int* crow, const int* col, const double* val, const double* x,
@@ -520,7 +571,15 @@ static void launch_spmv(int lanes, int grid, cudaStream_t s, long long n, const 
     case 208: FEMB_BSR(8) break;
     case 216: FEMB_BSR(16) break;
     case 232: FEMB_BSR(32) break;
-    case 101: FEMB_TMA(1) break;
+    case 101:
+      if (col16_hint) {
+        cudaFuncSetAttribute(spmv_tma16_kernel<FUSED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TMA16_SMEM);
+        launch_pdl(spmv_tma16_kernel<FUSED>, grid, TMA_THREADS, TMA16_SMEM, s, pdl_hint, n, nnz_hint, crow, col, val, x, y, mask, partial, st,
+                   eps, guards, rvec, tol, pin_hint, wvec, col16_hint, tile_ok_hint);
+      } else {
+        FEMB_TMA(1)
+      }
+      break;
     case 102: FEMB_TMA(2) break;
     case 104: FEMB_TMA(4) break;
     case 108: FEMB_TMA(8) break;
@@ -627,8 +686,42 @@ static int cg_solve_impl(int64_t n, int nmat, const CsrRef* mats, const double* 
   // two extra streamed vectors; FEMB_BSR_MERGED=1 selects the merged loop for A/B runs)
   static const bool bsr_merged = getenv("FEMB_BSR_MERGED") != nullptr;
   const bool merged = !classic_env && ((ll >= 300 && bsr_merged) || (ll >= 100 && ll < 200) || ll < 0);
+  // 16-bit delta-encoded column stream (DESIGN 3.4): the one-matrix merged loop on the LR = 1 TMA kernel, for solves of at
+  // least 16 iterations (the encode pass and its readback cost about 1 ms on C4, two and a half SpMVs).  Encoded on every call, so a pattern changed in place
+  // between two calls is always honoured; more than 1 % of tiles that do not encode -> the int32 kernel for the whole solve.
+  // FEMB_SPMV_IDX32=1 forces the int32 kernel (A/B runs).
+  static const bool idx32_env = getenv("FEMB_SPMV_IDX32") != nullptr;
+  bool use16 = !idx32_env && merged && nmat == 1 && lanes[0] == 101 && max_iter >= 16;
+  const long long ntiles16 = (n + TMA_THREADS - 1) / TMA_THREADS;
+  const size_t flags_off = 256, col16_off = flags_off + (((size_t)ntiles16 + 255) & ~(size_t)255);
+  if (use16) {
+    const size_t need16 = col16_off + 2 * (((size_t)mats[0].nnz + 7) & ~(size_t)7);  // padded: the last tile's copy stays in bounds
+    if (ctx->idx16_bytes < need16) {
+      if (ctx->graph_exec) cudaGraphExecDestroy(ctx->graph_exec), ctx->graph_exec = nullptr, ctx->graph_key_bytes = 0;
+      FEMB_CUDA(cudaStreamSynchronize(s));
+      if (ctx->idx16) cudaFree(ctx->idx16);
+      ctx->idx16 = nullptr, ctx->idx16_bytes = 0;
+      if (cudaMalloc(&ctx->idx16, need16) == cudaSuccess) ctx->idx16_bytes = need16;
+      else ctx->idx16 = nullptr, use16 = false, cudaGetLastError();  // out of memory: the int32 stream needs no extra bytes
+    }
+  }
+  if (use16) {
+    unsigned char* base16 = static_cast<unsigned char*>(ctx->idx16);
+    static_assert(2 * sizeof(CGState) + sizeof(int) <= 512 && 512 + sizeof(int) <= SOLVE_PINNED_BYTES, "pinned status buffer");
+    int* bad_host = reinterpret_cast<int*>(static_cast<unsigned char*>(ctx->pinned) + 512);
+    FEMB_CUDA(cudaMemsetAsync(base16, 0, sizeof(int), s));
+    idx16_encode_kernel<<<(int)std::min<long long>(ntiles16, (long long)SMS * 16), TMA_THREADS, 0, s>>>(
+        n, mats[0].crow, mats[0].col, reinterpret_cast<unsigned short*>(base16 + col16_off), base16 + flags_off, reinterpret_cast<int*>(base16));
+    FEMB_LAUNCH_CHECK();
+    FEMB_CUDA(cudaMemcpyAsync(bad_host, base16, sizeof(int), cudaMemcpyDeviceToHost, s));
+    FEMB_CUDA(cudaStreamSynchronize(s));
+    use16 = (long long)*bad_host * 100 <= ntiles16;
+  }
+  const unsigned short* col16 = use16 ? reinterpret_cast<const unsigned short*>(static_cast<unsigned char*>(ctx->idx16) + col16_off) : nullptr;
+  const unsigned char* tile_ok = use16 ? static_cast<unsigned char*>(ctx->idx16) + flags_off : nullptr;
   for (int m = 0; m < nmat; ++m) {
     g1[m] = spmv_grid(n, lanes[m], merged && m == nmat - 1);  // one grid per matrix: setup (plain) and loop (fused) launches share it
+    if (use16) g1[m] = tma16_grid(n);
     gmax = std::max(gmax, g1[m]);
   }
   const int g2 = grid_for(n, VEC_THREADS, 8);
@@ -649,8 +742,10 @@ static int cg_solve_impl(int64_t n, int nmat, const CsrRef* mats, const double* 
   double* partial = reinterpret_cast<double*>(static_cast<unsigned char*>(ctx->dev_scratch) + 256);
   // ---- setup (solver.py:163-181)
   if (mask) cg_mask_kernel<<<g2, VEC_THREADS, 0, s>>>(n, u, mask);
+  col16_hint = col16, tile_ok_hint = tile_ok;
   for (int m = 0; m < nmat; ++m)
     nnz_hint = mats[m].nnz, launch_spmv<false>(lanes[m], g1[m], s, n, mats[m].crow, mats[m].col, mats[m].val, u, Ap, nullptr, nullptr, nullptr, 0.0, m ? 2 : 0);
+  col16_hint = nullptr, tile_ok_hint = nullptr;
   cg_init_kernel<<<g2, VEC_THREADS, 0, s>>>(n, F, Ap, mask, minv, r, p, partial);
   cg_init_finish<<<1, VEC_THREADS, 0, s>>>(g2, partial, st, max_iter);
   FEMB_LAUNCH_CHECK();
@@ -664,12 +759,13 @@ static int cg_solve_impl(int64_t n, int nmat, const CsrRef* mats, const double* 
     const void *mask, *minv, *u, *work, *st, *partial;
     double tol, eps;
     long long pin;
+    const void* col16;
   } key;
   memset(&key, 0, sizeof(key));
   static_assert(sizeof(GraphKey) <= sizeof(ctx->graph_key), "graph key buffer");
   key.n = n, key.nmat = nmat, key.check_every = check_every, key.max_iter = max_iter, key.guards = guards, key.merged = merged ? 1 : 0;
   key.pdl = pdl_mode(), key.g2 = g2, key.g2v = g2v, key.mask = mask, key.minv = minv, key.u = u, key.work = work, key.st = st, key.partial = partial;
-  key.tol = tol, key.eps = eps, key.pin = spmv_pin_entries(mats[nmat - 1].nnz);
+  key.tol = tol, key.eps = eps, key.pin = spmv_pin_entries(mats[nmat - 1].nnz), key.col16 = col16;
   for (int m = 0; m < nmat; ++m) {
     key.lanes[m] = lanes[m], key.g1[m] = g1[m];
     key.nnz[m] = mats[m].nnz, key.crow[m] = mats[m].crow, key.col[m] = mats[m].col, key.val[m] = mats[m].val, key.block[m] = mats[m].block;
@@ -691,9 +787,10 @@ static int cg_solve_impl(int64_t n, int nmat, const CsrRef* mats, const double* 
       const bool pdl = pdl_enabled() && nmat == 1 && lanes[last] >= 100 && lanes[last] < 200;
       pdl_hint = pdl && k > 0 && (pdl_mode() & 2);
       pin_hint = pdl ? spmv_pin_entries(mats[last].nnz) : 0;
+      col16_hint = col16, tile_ok_hint = tile_ok;
       launch_spmv<true>(lanes[last], g1[last], s, n, mats[last].crow, mats[last].col, mats[last].val, p, Ap, mask, partial, st, eps,
                         guards | (last ? 2 : 0), r, tol, minv);
-      pdl_hint = false, pin_hint = 0;
+      pdl_hint = false, pin_hint = 0, col16_hint = nullptr, tile_ok_hint = nullptr;
       launch_pdl(cg_merged_kernel, g2v, VEC_THREADS, 0, s, pdl && (pdl_mode() & 1), n, u, r, p, Ap, minv, partial, st, max_iter, tol);
     } else {
       launch_spmv<true>(lanes[last], g1[last], s, n, mats[last].crow, mats[last].col, mats[last].val, p, Ap, mask, partial, st, eps,
@@ -756,6 +853,7 @@ static int cg_solve_impl(int64_t n, int nmat, const CsrRef* mats, const double* 
   result_host->status = fin->stop ? fin->status : 2;
   result_host->rs = fin->rs_new;
   result_host->loop_ms = ms;
+  result_host->index_bytes = use16 ? 2 : 4;
   return FEMB_OK;
 }
 
@@ -897,5 +995,6 @@ extern "C" int femb_cg_solve_operator(int64_t n, femb_apply_fn apply, void* ctx,
   result_host->status = h.stop ? h.status : 2;
   result_host->rs = h.rs_new;
   result_host->loop_ms = ms;
+  result_host->index_bytes = 0;  // the operator is the caller's callback
   return FEMB_OK;
 }

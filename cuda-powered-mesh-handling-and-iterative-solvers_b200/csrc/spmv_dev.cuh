@@ -384,6 +384,168 @@ inline int tma_grid(long long n, int lr) {
   return (int)std::max<long long>(1, std::min<long long>(tiles, (long long)SMS * TMA_CTAS_PER_SM));
 }
 
+// IDX16 variant (LR = 1): 10 bytes per staged entry.  A full 128-row tile of the P1 Kuhn-cube operator (15 nonzeros per row)
+// needs 1927 entries with the 8-entry alignment.  The -D overrides exist for the stage / CTA sweep (DESIGN 3.4).
+#ifndef FEMB_TMA16_STAGES
+#define FEMB_TMA16_STAGES 2
+#endif
+#ifndef FEMB_TMA16_CAP
+#define FEMB_TMA16_CAP 2176
+#endif
+#ifndef FEMB_TMA16_CTAS
+#define FEMB_TMA16_CTAS 5
+#endif
+constexpr int TMA16_STAGES = FEMB_TMA16_STAGES, TMA16_CAP = FEMB_TMA16_CAP, TMA16_CTAS_PER_SM = FEMB_TMA16_CTAS;
+constexpr size_t TMA16_SMEM = (size_t)TMA16_STAGES * TMA16_CAP * 10;
+inline int tma16_grid(long long n) {
+  const long long tiles = (n + TMA_THREADS - 1) / TMA_THREADS;
+  return (int)std::max<long long>(1, std::min<long long>(tiles, (long long)SMS * TMA16_CTAS_PER_SM));
+}
+
+// 16-bit-index twin of spmv_tma_rows<1, true, ..., NoHaloWait, PdlWait> for the merged CG loop (a sibling, so the int32 kernels
+// of krylov.cu and dist.cu compile exactly as before).  The staged index stream is col16 (idx16_encode_kernel, krylov.cu):
+// col16[a] = r - col[a] for the first entry a of row r, col16[j] = col[j] - col[j-1] after it, i.e. 10 instead of 12 bytes per
+// staged nonzero.  One lane owns a row and rebuilds its columns with one running add per entry; the products are summed in the
+// int32 kernel's order, so y is bit-identical.  A tile whose tile_ok byte is 0, that does not fit a stage, or whose val copy
+// would run past nnz (col16 itself is padded) takes the direct path from the int32 col.  Slices start at a multiple of 8
+// entries (16-byte aligned 2-byte copy); val is copied in pairs of entries.
+template <int STAGES, int CAP>
+__device__ __forceinline__ double spmv_tma16_rows(long long n, long long nnz, const int* __restrict__ crow, const int* __restrict__ col,
+                                                  const unsigned short* __restrict__ col16, const unsigned char* __restrict__ tile_ok,
+                                                  const double* __restrict__ val, const double* __restrict__ x, double* __restrict__ y,
+                                                  const unsigned char* __restrict__ mask, bool accumulate, bool fused,
+                                                  const double* __restrict__ rvec, double* extra, const int* stop, long long pin,
+                                                  const double* __restrict__ wvec) {
+  static_assert(CAP % 8 == 0, "16-byte aligned stages");
+  constexpr int R = TMA_THREADS;
+  extern __shared__ __align__(128) unsigned char tma_smem[];
+  double* vbuf = reinterpret_cast<double*>(tma_smem);                                                 // [STAGES][CAP]
+  unsigned short* dbuf = reinterpret_cast<unsigned short*>(tma_smem + sizeof(double) * STAGES * CAP);  // [STAGES][CAP]
+  __shared__ unsigned long long full[STAGES];
+  __shared__ int base[STAGES];  // first staged entry of the tile (aligned down), -1 = not staged (direct path)
+  const int tid = threadIdx.x;
+  const long long ntiles = (n + R - 1) / R;
+  const bool use_hint = g_spmv_l2_hint != 0;
+  const unsigned long long pol = l2_evict_first_policy(), pol_keep = l2_evict_last_policy();
+  if (tid == 0) {
+    for (int s = 0; s < STAGES; ++s) mbar_init(&full[s], 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  __syncthreads();
+  // producer (thread 0): row-pointer pair and flag of the tile it stages next are requested one iteration early
+  auto bounds = [&](long long k, int& a, int& b, int& ok) {
+    const long long t = blockIdx.x + k * gridDim.x;
+    a = b = ok = 0;
+    if (t < ntiles) a = __ldg(crow + t * R), b = __ldg(crow + min(n, t * R + R)), ok = __ldg(tile_ok + t);
+  };
+  auto stage_tile = [&](long long k, int a, int b, int ok) {
+    if (blockIdx.x + k * gridDim.x >= ntiles) return;
+    const int s = (int)(k % STAGES);
+    const int a0 = a & ~7, cnt = (b - a0 + 7) & ~7, cntv = (b - a0 + 1) & ~1;
+    if (!ok || cnt > CAP || (long long)a0 + cntv > nnz || b == a) {
+      base[s] = -1;
+      return;
+    }
+    base[s] = a0;
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    mbar_expect_tx(&full[s], (unsigned)cntv * 8u + (unsigned)cnt * 2u);
+    if (use_hint) {
+      const unsigned long long pl = (long long)a0 + cntv <= pin ? pol_keep : pol;
+      bulk_g2s_hint(vbuf + (size_t)s * CAP, val + a0, (unsigned)cntv * 8u, &full[s], pl);
+      bulk_g2s_hint(dbuf + (size_t)s * CAP, col16 + a0, (unsigned)cnt * 2u, &full[s], pl);
+    } else {
+      bulk_g2s(vbuf + (size_t)s * CAP, val + a0, (unsigned)cntv * 8u, &full[s]);
+      bulk_g2s(dbuf + (size_t)s * CAP, col16 + a0, (unsigned)cnt * 2u, &full[s]);
+    }
+  };
+  int na = 0, nb = 0, nok = 0;
+  if (tid == 0) {
+    for (int k = 0; k < STAGES - 1; ++k) {
+      bounds(k, na, nb, nok);
+      stage_tile(k, na, nb, nok);
+    }
+    bounds(STAGES - 1, na, nb, nok);
+  }
+  double dot = 0.0;
+  unsigned phase_bits = 0;
+  pdl_wait();  // everything above touched only the matrix; x, y, rvec may come from the previous kernel
+  if (stop) {  // sticky stop flag: drain what was staged, then leave
+    __shared__ int stop_sh;
+    if (tid == 0) stop_sh = *(volatile const int*)stop;
+    __syncthreads();
+    if (stop_sh) {
+      for (int k = 0; k < STAGES - 1; ++k)
+        if (blockIdx.x + (long long)k * gridDim.x < ntiles && base[k % STAGES] >= 0) mbar_wait(&full[k % STAGES], 0u);
+      return 0.0;
+    }
+  }
+  for (long long k = 0;; ++k) {
+    const long long t = blockIdx.x + k * gridDim.x;
+    if (t >= ntiles) break;
+    const int s = (int)(k % STAGES);
+    if (tid == 0) {
+      stage_tile(k + STAGES - 1, na, nb, nok);
+      bounds(k + STAGES, na, nb, nok);
+    }
+    const long long r = t * R + tid;
+    int ra = 0, rb = 0;
+    double x_own = 0.0, y_prev = 0.0, r_own = 0.0, w_own = 1.0;
+    bool keep = true;
+    if (r < n) {
+      ra = __ldg(crow + r), rb = __ldg(crow + r + 1);
+      if (fused) {
+        x_own = __ldg(x + r);
+        if (mask) keep = mask[r] != 0;
+        if (rvec) r_own = rvec[r];
+        if (wvec) w_own = wvec[r];
+      }
+      if (accumulate) y_prev = y[r];
+    }
+    __syncthreads();  // base[s] written by thread 0 is visible
+    const int a0 = base[s];
+    double sum = 0.0;
+    if (a0 >= 0) {
+      mbar_wait(&full[s], (phase_bits >> s) & 1u);
+      phase_bits ^= 1u << s;
+      const double* vs = vbuf + (size_t)s * CAP - a0;
+      const unsigned short* ds = dbuf + (size_t)s * CAP - a0;
+      int c = ra < rb ? (int)r - 2 * (int)ds[ra] : 0;  // + ds[ra] = the first column
+      int j = ra;
+      for (; j + 7 < rb; j += 8) {  // eight independent x gathers in flight
+        double xv[8];
+#pragma unroll
+        for (int q = 0; q < 8; ++q) c += ds[j + q], xv[q] = __ldg(x + c);
+#pragma unroll
+        for (int q = 0; q < 8; ++q) sum += vs[j + q] * xv[q];
+      }
+      {  // tail: up to seven more, still issued together
+        double xv[7];
+#pragma unroll
+        for (int q = 0; q < 7; ++q) {
+          if (j + q < rb) c += ds[j + q];
+          xv[q] = (j + q < rb) ? __ldg(x + c) : 0.0;
+        }
+#pragma unroll
+        for (int q = 0; q < 7; ++q)
+          if (j + q < rb) sum += vs[j + q] * xv[q];
+      }
+    } else {
+      for (int j = ra; j < rb; ++j) sum += ld_stream(val + j) * __ldg(x + ld_stream(col + j));
+    }
+    if (r < n) {
+      if (accumulate) sum += y_prev;
+      if (fused) {
+        if (!keep) sum = 0.0;
+        dot += sum * x_own;
+        if (extra) extra[0] += sum * (w_own * r_own), extra[1] += sum * (sum * w_own);
+      }
+      y[r] = sum;
+    }
+    __syncthreads();  // the stage is drained: thread 0 may refill it in the next iteration
+  }
+  return dot;
+}
+
 // ---- TMA-pipelined block-CSR SpMV, 3x3 blocks (elasticity: 3 dofs per node) ---------------------------------------------------
 // The node-level pattern (brow/bcol) with one 72-byte row-major block per entry cuts the index stream 9x against scalar CSR
 // (12 -> 8.44 bytes per scalar nonzero) and fetches x[3c..3c+2] once per block instead of once per scalar row, i.e. a third

@@ -15,7 +15,8 @@ c_i32, c_i64, c_f64, c_vp = C.c_int, C.c_int64, C.c_double, C.c_void_p
 
 
 class CGResult(C.Structure):
-    _fields_ = [("iterations", C.c_int32), ("status", C.c_int32), ("rs", C.c_double), ("loop_ms", C.c_double)]
+    _fields_ = [("iterations", C.c_int32), ("status", C.c_int32), ("rs", C.c_double), ("loop_ms", C.c_double),
+                ("index_bytes", C.c_int32)]
 
 
 # int (*femb_apply_fn)(void* ctx, const double* x, double* y, femb_stream stream)

@@ -594,7 +594,8 @@ def cg_solve(crow, col, val, F, mask=None, minv=None, u_init=None, tol=1e-10, ma
     with torch.cuda.device(dev):
         check(lib.femb_cg_solve(n, val.numel(), _p(crow), _p(col), _p(val), _p(Ff), _p(mask), _p(minv), _p(u), _p(work), float(tol),
                                 int(max_iter), float(eps), int(check_every), C.byref(res), _stream(dev)), "femb_cg_solve")
-    info = {"iterations": res.iterations, "status": STATUS.get(res.status, "?"), "rs": res.rs, "loop_ms": res.loop_ms}
+    info = {"iterations": res.iterations, "status": STATUS.get(res.status, "?"), "rs": res.rs, "loop_ms": res.loop_ms,
+            "index_bytes": res.index_bytes}
     return u.reshape(F.shape), info
 
 

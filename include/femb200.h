@@ -260,6 +260,7 @@ typedef struct femb_cg_result {
   int32_t status;     /* 0 converged, 1 breakdown (pAp guard / NaN), 2 max_iter */
   double rs;          /* last r.r (or r.z) */
   double loop_ms;     /* device time of the iteration loop (CUDA events on the solver stream) */
+  int32_t index_bytes; /* bytes per column index the loop's SpMV streamed: 2 = 16-bit delta-encoded, 4 = int32 CSR */
 } femb_cg_result;
 
 /* stable_conjugate_gradient_solver solver.py:144-229 (also the loops of :11-135, :231-295, :297-389) on the
