@@ -10,6 +10,10 @@
 //                    coefficients without repeating an SpMM
 //   lobpcg_residual  R = KX - MX diag(lam), per-column |r|^2 and |x|^2 (deterministic), W = D^-1 R for the active columns
 // The 3m x 3m Rayleigh-Ritz problems run on the host.
+// Two more kernels make up the V-cycle preconditioner of subdivided_lowest_modes (femb200/multigrid.py), on the same layout:
+//   mg_smooth        one damped-Jacobi step X_out = X_in + omega dinv (R - A X_in) and/or the residual R - A X_in, on the SpMM's
+//                    block traversal (each 3x3 block of A read once for all m columns)
+//   mg_transfer      Y (+)= mask (S (x) I3) X for a node-level scalar CSR S: the prolongation P and the restriction R = P^T
 #include "common.cuh"
 #include "spmv_dev.cuh"
 
@@ -42,12 +46,13 @@ __device__ __forceinline__ int ld_stream(const int* p, unsigned long long pol) {
 // slot = lane / mp one of 32/mp blocks handled side by side; lanes of one slot load the same 3x3 block (one uniform-address
 // load), lanes of one column load x rows that are contiguous across c.  The matrix stream carries an L2 evict-first hint: it is
 // read once per SpMM and should not push the multivectors out of L2.  Slots are summed by a fixed xor tree (deterministic).
-template <bool HAS_M>
-__global__ void __launch_bounds__(MB_THREADS) spmm_bsr3_kernel(long long nb, const int* __restrict__ brow, const int* __restrict__ bcol,
-                                                                const double* __restrict__ kval, const double* __restrict__ mval,
-                                                                const unsigned char* __restrict__ mask, int m, int log_mp,
-                                                                const double* __restrict__ X, long long ldx, double* __restrict__ YK,
-                                                                double* __restrict__ YM, long long ldy) {
+// The traversal is shared by the SpMM and the multigrid smoother (mg_smooth_kernel below); the lane (slot 0, column c) of each row
+// hands its three row sums of K X (and M X) to the epilogue: epi(row, c, k0, k1, k2, m0, m1, m2).
+template <bool HAS_M, class Epi>
+__device__ __forceinline__ void bsr3_warp_rows(long long nb, const int* __restrict__ brow, const int* __restrict__ bcol,
+                                               const double* __restrict__ kval, const double* __restrict__ mval,
+                                               const unsigned char* __restrict__ mask, int m, int log_mp, const double* __restrict__ X,
+                                               long long ldx, Epi epi) {
   const unsigned long long pol = l2_evict_first_policy();
   const int lane = threadIdx.x & 31;
   const int mp = 1 << log_mp;
@@ -92,20 +97,30 @@ __global__ void __launch_bounds__(MB_THREADS) spmm_bsr3_kernel(long long nb, con
         m2 += __shfl_xor_sync(0xffffffffu, m2, o);
       }
     }
-    if (slot == 0 && col_ok) {
-      const bool f0 = !mask || mask[3 * row], f1 = !mask || mask[3 * row + 1], f2 = !mask || mask[3 * row + 2];
-      double* yk = YK + 3 * row * ldy + c;
-      yk[0] = f0 ? k0 : 0.0;
-      yk[ldy] = f1 ? k1 : 0.0;
-      yk[2 * ldy] = f2 ? k2 : 0.0;
-      if (HAS_M) {
-        double* ym = YM + 3 * row * ldy + c;
-        ym[0] = f0 ? m0 : 0.0;
-        ym[ldy] = f1 ? m1 : 0.0;
-        ym[2 * ldy] = f2 ? m2 : 0.0;
-      }
-    }
+    if (slot == 0 && col_ok) epi(row, c, k0, k1, k2, m0, m1, m2);
   }
+}
+
+template <bool HAS_M>
+__global__ void __launch_bounds__(MB_THREADS) spmm_bsr3_kernel(long long nb, const int* __restrict__ brow, const int* __restrict__ bcol,
+                                                                const double* __restrict__ kval, const double* __restrict__ mval,
+                                                                const unsigned char* __restrict__ mask, int m, int log_mp,
+                                                                const double* __restrict__ X, long long ldx, double* __restrict__ YK,
+                                                                double* __restrict__ YM, long long ldy) {
+  bsr3_warp_rows<HAS_M>(nb, brow, bcol, kval, mval, mask, m, log_mp, X, ldx,
+                        [&](long long row, int c, double k0, double k1, double k2, double m0, double m1, double m2) {
+                          const bool f0 = !mask || mask[3 * row], f1 = !mask || mask[3 * row + 1], f2 = !mask || mask[3 * row + 2];
+                          double* yk = YK + 3 * row * ldy + c;
+                          yk[0] = f0 ? k0 : 0.0;
+                          yk[ldy] = f1 ? k1 : 0.0;
+                          yk[2 * ldy] = f2 ? k2 : 0.0;
+                          if (HAS_M) {
+                            double* ym = YM + 3 * row * ldy + c;
+                            ym[0] = f0 ? m0 : 0.0;
+                            ym[ldy] = f1 ? m1 : 0.0;
+                            ym[2 * ldy] = f2 ? m2 : 0.0;
+                          }
+                        });
 }
 
 // G = A^T B: a tile of GR_ROWS rows of A and B (zero-padded to 48 columns) is staged in shared memory; thread (bi, bj) of a
@@ -206,6 +221,77 @@ __global__ void __launch_bounds__(MB_THREADS) lobpcg_residual_kernel(long long n
     double s = 0.0;
     for (int y = 0; y < MB_THREADS / 16; ++y) s += red[w][y][c];
     partial[(size_t)blockIdx.x * (2 * m) + threadIdx.x] = s;
+  }
+}
+
+// One damped-Jacobi step on m columns: t = mask (R - A X_in), Res = t and X_out = X_in + omega dinv t (each output optional).
+// HAS_X = false is X_in = 0: t = mask R and the matrix is not read, so the lanes of slot 0 of each warp cover the rows directly.
+template <bool HAS_X>
+__global__ void __launch_bounds__(MB_THREADS) mg_smooth_kernel(long long nb, const int* __restrict__ brow, const int* __restrict__ bcol,
+                                                                const double* __restrict__ aval, const unsigned char* __restrict__ mask,
+                                                                const double* __restrict__ dinv, double omega, int m, int log_mp,
+                                                                const double* __restrict__ R, long long ldr, const double* __restrict__ X,
+                                                                long long ldx, double* __restrict__ Xo, long long ldo, double* __restrict__ Res,
+                                                                long long ldres) {
+  auto epi = [&](long long row, int c, double a0, double a1, double a2, double, double, double) {
+    const double a[3] = {a0, a1, a2};
+#pragma unroll
+    for (int d = 0; d < 3; ++d) {
+      const long long r = 3 * row + d;
+      const double t = (!mask || mask[r]) ? R[r * ldr + c] - a[d] : 0.0;
+      if (Res) Res[r * ldres + c] = t;
+      if (Xo) Xo[r * ldo + c] = (HAS_X ? X[r * ldx + c] : 0.0) + omega * dinv[r] * t;
+    }
+  };
+  if (HAS_X) {
+    bsr3_warp_rows<false>(nb, brow, bcol, aval, nullptr, mask, m, log_mp, X, ldx, epi);
+  } else {
+    const int c = threadIdx.x & 31;
+    const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
+    if (c < m)
+      for (long long row = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; row < nb; row += nwarps) epi(row, c, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0);
+  }
+}
+
+// Y[3i+d, j] (+)= mask_out[3i+d] sum_k val[k] X[3 col[k]+d, j] for a node-level scalar CSR (the prolongation or the restriction):
+// one warp per output node, lanes (slot, c) as in the SpMM, slots over the row's entries, summed by the same fixed xor tree.
+__global__ void __launch_bounds__(MB_THREADS) mg_transfer_kernel(long long n_out, const int* __restrict__ crow, const int* __restrict__ col,
+                                                                  const double* __restrict__ val, const unsigned char* __restrict__ mask_out,
+                                                                  int m, int log_mp, const double* __restrict__ X, long long ldx, int accumulate,
+                                                                  double* __restrict__ Y, long long ldy) {
+  const int lane = threadIdx.x & 31;
+  const int mp = 1 << log_mp;
+  const int c = lane & (mp - 1), slot = lane >> log_mp, nslot = 32 >> log_mp;
+  const bool col_ok = c < m;
+  const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
+  for (long long row = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; row < n_out; row += nwarps) {
+    const int k0 = __ldg(crow + row), k1 = __ldg(crow + row + 1);
+    double s0 = 0.0, s1 = 0.0, s2 = 0.0;
+    for (int k = k0 + slot; k < k1; k += nslot) {
+      const long long j = __ldg(col + k);
+      const double v = __ldg(val + k);
+      if (col_ok) {
+        const double* xp = X + 3 * j * ldx + c;
+        s0 += v * xp[0];
+        s1 += v * xp[ldx];
+        s2 += v * xp[2 * ldx];
+      }
+    }
+    for (int o = mp; o < 32; o <<= 1) {
+      s0 += __shfl_xor_sync(0xffffffffu, s0, o);
+      s1 += __shfl_xor_sync(0xffffffffu, s1, o);
+      s2 += __shfl_xor_sync(0xffffffffu, s2, o);
+    }
+    if (slot == 0 && col_ok) {
+      const double s[3] = {s0, s1, s2};
+#pragma unroll
+      for (int d = 0; d < 3; ++d) {
+        const long long r = 3 * row + d;
+        const double v = (!mask_out || mask_out[r]) ? s[d] : 0.0;
+        double* y = Y + r * ldy + c;
+        *y = accumulate ? *y + v : v;
+      }
+    }
   }
 }
 
@@ -314,6 +400,50 @@ extern "C" int femb_lobpcg_residual(int64_t n, int m, const double* X, int64_t l
   FEMB_CUDA(scr.alloc(&partial, (size_t)grid * 2 * m));
   lobpcg_residual_kernel<<<grid, MB_THREADS, 0, s>>>(n, m, X, ldx, KX, MX, ldk, lam, dinv, na, active, W, ldw, partial);
   mb_partial_finish<<<1, MB_THREADS, 0, s>>>(grid, 2 * m, partial, norms);
+  FEMB_LAUNCH_CHECK();
+  return FEMB_OK;
+}
+
+extern "C" int femb_mg_smooth_bsr3(int64_t nb, int64_t nnzb, const int32_t* brow, const int32_t* bcol, const double* aval, const uint8_t* mask,
+                                   const double* dinv, double omega, int m, const double* R, int64_t ldr, const double* X_in, int64_t ldx,
+                                   double* X_out, int64_t ldo, double* Res, int64_t ldres, femb_stream stream) {
+  FEMB_CHECK_ARG(m >= 1 && m <= MB_MAXM, "1 <= m <= 16");
+  FEMB_CHECK_ARG(nb >= 0 && nnzb >= 0 && nnzb <= INT32_MAX, "nb >= 0, 0 <= nnzb < 2^31");
+  FEMB_CHECK_ARG(brow && bcol && aval && R && (X_out || Res) && (!X_out || dinv),
+                 "non-null brow, bcol, aval, R, at least one of X_out and Res (and dinv with X_out)");
+  FEMB_CHECK_ARG(ldr >= m && (!X_in || ldx >= m) && (!X_out || ldo >= m) && (!Res || ldres >= m), "ldr, ldx, ldo, ldres >= m");
+  const long long n = 3 * nb;
+  const bool bad = (X_out && X_in && views_overlap(X_out, ldo, m, X_in, ldx, m, n)) || (X_out && views_overlap(X_out, ldo, m, R, ldr, m, n)) ||
+                   (Res && X_in && views_overlap(Res, ldres, m, X_in, ldx, m, n)) || (Res && views_overlap(Res, ldres, m, R, ldr, m, n)) ||
+                   (X_out && Res && views_overlap(X_out, ldo, m, Res, ldres, m, n));
+  FEMB_CHECK_ARG(!bad, "outputs overlap the inputs or each other");
+  if (nb == 0) return FEMB_OK;
+  cudaStream_t s = as_stream(stream);
+  int log_mp = 0;
+  while ((1 << log_mp) < m) ++log_mp;
+  const int grid = grid_for(nb * 32, MB_THREADS, 32);
+  if (X_in)
+    mg_smooth_kernel<true><<<grid, MB_THREADS, 0, s>>>(nb, brow, bcol, aval, mask, dinv, omega, m, log_mp, R, ldr, X_in, ldx, X_out, ldo, Res, ldres);
+  else
+    mg_smooth_kernel<false><<<grid, MB_THREADS, 0, s>>>(nb, brow, bcol, aval, mask, dinv, omega, m, log_mp, R, ldr, nullptr, 0, X_out, ldo, Res, ldres);
+  FEMB_LAUNCH_CHECK();
+  return FEMB_OK;
+}
+
+extern "C" int femb_mg_transfer(int64_t n_out, int64_t n_in, int64_t nnz, const int32_t* crow, const int32_t* col, const double* val,
+                                const uint8_t* mask_out, int m, const double* X, int64_t ldx, int accumulate, double* Y, int64_t ldy,
+                                femb_stream stream) {
+  FEMB_CHECK_ARG(m >= 1 && m <= MB_MAXM, "1 <= m <= 16");
+  FEMB_CHECK_ARG(n_out >= 0 && n_in >= 0 && nnz >= 0 && nnz <= INT32_MAX, "n_out, n_in >= 0, 0 <= nnz < 2^31");
+  FEMB_CHECK_ARG(crow && col && val && X && Y, "non-null crow, col, val, X, Y");
+  FEMB_CHECK_ARG(ldx >= m && ldy >= m, "ldx, ldy >= m");
+  FEMB_CHECK_ARG(accumulate == 0 || accumulate == 1, "accumulate is 0 or 1");
+  FEMB_CHECK_ARG(n_in == 0 || n_out == 0 || !spans_meet(Y, (3 * n_out - 1) * ldy + m, X, (3 * n_in - 1) * ldx + m), "Y overlaps X");
+  if (n_out == 0) return FEMB_OK;
+  int log_mp = 0;
+  while ((1 << log_mp) < m) ++log_mp;
+  mg_transfer_kernel<<<grid_for(n_out * 32, MB_THREADS, 32), MB_THREADS, 0, as_stream(stream)>>>(n_out, crow, col, val, mask_out, m, log_mp, X, ldx,
+                                                                                                accumulate, Y, ldy);
   FEMB_LAUNCH_CHECK();
   return FEMB_OK;
 }

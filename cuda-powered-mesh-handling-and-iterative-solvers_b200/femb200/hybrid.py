@@ -63,6 +63,17 @@ def _restriction_csr(parents, n_coarse, dev):
     return crow.to(torch.int32).contiguous(), cols.to(torch.int32).contiguous(), vals.contiguous()
 
 
+def _prolongation_csr(parents, n_coarse, dev):
+    """P as CSR [n_coarse + n_mid, n_coarse], the matrix of `prolongate`: row i < n_coarse holds (i, 1), row n_coarse + k holds
+    (parents[k], 1/2) with the two columns ascending."""
+    nm = parents.shape[0]
+    pc = torch.sort(parents, dim=1).values
+    cols = torch.cat([torch.arange(n_coarse, device=dev), pc.reshape(-1)])
+    vals = torch.cat([torch.ones(n_coarse, device=dev, dtype=torch.float64), torch.full((2 * nm,), 0.5, device=dev, dtype=torch.float64)])
+    crow = torch.cat([torch.arange(n_coarse + 1, device=dev), n_coarse + 2 * torch.arange(1, nm + 1, device=dev)])
+    return crow.to(torch.int32).contiguous(), cols.to(torch.int32).contiguous(), vals.contiguous()
+
+
 def multilevel_solve(coords, tets, levels, load_fn, fixed_fn, E=None, nu=None, kind="elasticity", tol=1e-8, max_iter=500, device="cuda:0",
                      element_module=None, verbose=False, smooth=2, omega=0.6):
     """CG on the finest mesh preconditioned by a V(smooth, smooth) cycle over the hierarchy coarse mesh + `levels` uniform

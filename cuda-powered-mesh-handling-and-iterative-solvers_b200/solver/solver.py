@@ -556,6 +556,40 @@ def lowest_modes(K_local, M_local, elements, fixed, num_nodes, num_eigs=6, tol=1
     return (lam, modes_out, info) if return_info else (lam, modes_out)
 
 
+def subdivided_lowest_modes(coords, elements, levels, fixed_fn, E, nu, rho, num_eigs=6, tol=1e-8, max_iter=500, shift=0.0, device="cuda:0",
+                            dtype=torch.float64, return_info=False, verbose=True):
+    """Lowest eigenpairs of K x = lam M x on a refined C3D4 mesh (not in the reference): the coarse mesh (coords, elements) is refined
+    `levels` times as in hybrid_subdivided_solver, K (E, nu) and the consistent M (rho) are assembled on every level, and LOBPCG on
+    the finest mesh is preconditioned by a V-cycle over the hierarchy (femb200/multigrid.py) instead of Jacobi, so the iteration
+    count stays roughly flat as the mesh is refined.  fixed_fn(coords_l) -> clamped node ids (all three dofs) on every level.
+    The result is what lowest_modes returns on the finest mesh, within tol (same backward-error test, M-orthonormal modes, zeros on
+    fixed dofs).  `shift` >= 0: the preconditioner approximates (K + shift M)^-1; 0 suits any clamped model, a free-free model needs
+    shift > 0 (a ValueError says so when the coarse K + shift M is singular).  The coarse mesh may hold at most
+    multigrid.MAX_COARSE_DOFS free dofs (dense factor).  1 <= num_eigs <= 12.
+    Returns (lam [num_eigs], modes [3*N_fine, num_eigs], coords_fine, elements_fine), lam and modes cast to `dtype`; with
+    return_info also the dict of lowest_modes plus `levels` (nodes, tets, dofs per level, coarsest first) and `shift`."""
+    from femb200 import modes, multigrid
+    dev = _ops.cuda_device(device)
+    if not 1 <= num_eigs <= 12:
+        raise ValueError("num_eigs must be between 1 and 12")
+    if not shift >= 0.0:
+        raise ValueError("shift must be >= 0")
+    if int(levels) != levels or levels < 0:
+        raise ValueError("levels must be a non-negative integer")
+    H = multigrid.Hierarchy(coords, elements, int(levels), fixed_fn, E, nu, rho, shift, dev, _el)
+    lam, S, info = modes.lobpcg(multigrid.MultilevelBackend(H), num_eigs, tol=tol, max_iter=max_iter)
+    info["levels"], info["shift"] = H.describe(), float(shift)
+    if verbose:
+        if info["status"] == "converged":
+            print(f"Multigrid LOBPCG converged after {info['iterations']} iterations on {H.L[-1].n} dofs ({len(H.L)} levels).")
+        else:
+            print(f"Multigrid LOBPCG did not converge within {max_iter} iterations; max residual {info['residuals'].max():.3e}.")
+    lam = torch.from_numpy(lam).to(device=dev, dtype=dtype)
+    modes_out = S[:, :num_eigs].contiguous().to(dtype)
+    out = (lam, modes_out, H.coords, H.tets)
+    return out + (info,) if return_info else out
+
+
 def static_structure_solver(coords, force, fixed, c3d4=None, c3d6=None, c3d8=None, s3=None, s4=None, material=None, u_init=None,
                             tol=1e-10, max_iter=1000, device="cuda:0", dtype=torch.float64, eps=1e-30, return_info=False, verbose=True):
     """Mixed-element static solve on [N,6] (solver.py:11-135): solids act on the translations, shells on all six dofs

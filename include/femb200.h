@@ -321,6 +321,19 @@ int femb_lobpcg_residual(int64_t n, int m, const double* X, int64_t ldx, const d
                          const double* lam_host, const double* dinv, int na, const int32_t* active, double* W, int64_t ldw,
                          double* norms, femb_stream stream);
 
+/* Multigrid V-cycle kernels of subdivided_lowest_modes (same multivector layout and rules as the block kernels above).
+ *   femb_mg_smooth_bsr3: t = mask (R - A X_in) on 1 <= m <= 16 columns (A: 3x3 block-CSR as in femb_spmm_bsr3, x masked as there;
+ *     mask NULL: none); Res = t and X_out = X_in + omega dinv t, each optional (at least one given; dinv [3 nb] needed with X_out).
+ *     X_in NULL means X_in = 0 (X_out = omega dinv mask R, the matrix is not read).  X_out must not overlap X_in: ping-pong.
+ *   femb_mg_transfer: Y[3i+d, j] (+)= mask_out[3i+d] sum_k val[k] X[3 col[k]+d, j] for the node-level scalar CSR (crow [n_out+1],
+ *     col [nnz] < n_in, int32; val fp64) -- the prolongation or the restriction; accumulate = 1 adds to Y, 0 overwrites it. */
+int femb_mg_smooth_bsr3(int64_t nb, int64_t nnzb, const int32_t* brow, const int32_t* bcol, const double* aval, const uint8_t* mask,
+                        const double* dinv, double omega, int m, const double* R, int64_t ldr, const double* X_in, int64_t ldx,
+                        double* X_out, int64_t ldo, double* Res, int64_t ldres, femb_stream stream);
+int femb_mg_transfer(int64_t n_out, int64_t n_in, int64_t nnz, const int32_t* crow, const int32_t* col, const double* val,
+                     const uint8_t* mask_out, int m, const double* X, int64_t ldx, int accumulate, double* Y, int64_t ldy,
+                     femb_stream stream);
+
 /* Jacobi diagonal of a CSR matrix: minv[i] = mask[i] ? 1/A_ii : 0 (the documented replacement for the
  * reference's broken compute_diagonal_preconditioner solver.py:814-833) */
 int femb_csr_jacobi(int64_t n, const int32_t* crow, const int32_t* col, const double* val, const uint8_t* mask,
