@@ -20,7 +20,8 @@ struct Tet {
 };
 
 template <typename T, typename I>
-__device__ __forceinline__ void tet_setup(const T* __restrict__ coords, const I* __restrict__ conn, long long e, Tet<T>& t) {
+__device__ __forceinline__ void tet_setup(const T* __restrict__ coords, const I* __restrict__ conn, long long e, Tet<T>& t,
+                                          long long* ids = nullptr) {
   long long n[4];
   if (sizeof(I) == 8) {  // one 256-bit load of the element's four int64 ids
     asm volatile("ld.global.nc.L1::no_allocate.v4.s64 {%0,%1,%2,%3}, [%4];" : "=l"(n[0]), "=l"(n[1]), "=l"(n[2]), "=l"(n[3]) : "l"(conn + 4 * e));
@@ -28,6 +29,9 @@ __device__ __forceinline__ void tet_setup(const T* __restrict__ coords, const I*
     const int4 q = __ldg(reinterpret_cast<const int4*>(conn) + e);
     n[0] = q.x, n[1] = q.y, n[2] = q.z, n[3] = q.w;
   }
+  if (ids)
+#pragma unroll
+    for (int a = 0; a < 4; ++a) ids[a] = n[a];
   T x[4][3];
 #pragma unroll
   for (int a = 0; a < 4; ++a)
@@ -178,6 +182,53 @@ static int c3d4_dispatch(int what, const void* coords, const void* conn, long lo
   }
   FEMB_LAUNCH_CHECK();
   return FEMB_OK;
+}
+
+// Geometric stiffness of the stress of a displacement field (not in the reference), one thread per element.  The strain is
+// constant on a C3D4, so H = sum_a g_a (x) u_a, sigma = lam tr(H) I + mu (H + H^T) and s_ab = V g_a^T sigma g_b are formed in
+// registers; block (a,b) of the [12,12] output is s_ab I3.  s_ab is computed once for a <= b and mirrored (bitwise symmetric).
+template <typename T, typename I>
+__global__ void __launch_bounds__(128) c3d4_geometric_kernel(const T* __restrict__ coords, const I* __restrict__ conn, long long M,
+                                                             const T* __restrict__ disp, T lam, T mu, T* __restrict__ out) {
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < M; e += (long long)gridDim.x * blockDim.x) {
+    Tet<T> t;
+    long long n[4];
+    tet_setup(coords, conn, e, t, n);
+    T H[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};  // H[i][k] = du_k / dx_i
+#pragma unroll
+    for (int a = 0; a < 4; ++a) {
+      const T u[3] = {__ldg(disp + 3 * n[a]), __ldg(disp + 3 * n[a] + 1), __ldg(disp + 3 * n[a] + 2)};
+#pragma unroll
+      for (int i = 0; i < 3; ++i)
+#pragma unroll
+        for (int k = 0; k < 3; ++k) H[3 * i + k] += t.g[a][i] * u[k];
+    }
+    const T V = fabs(t.det) / T(6), tr = lam * (H[0] + H[4] + H[8]);
+    T sig[9];
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+      for (int k = 0; k < 3; ++k) sig[3 * i + k] = V * (mu * (H[3 * i + k] + H[3 * k + i]) + (i == k ? tr : T(0)));
+    T s[4][4];
+#pragma unroll
+    for (int b = 0; b < 4; ++b) {
+      const T sg[3] = {sig[0] * t.g[b][0] + sig[1] * t.g[b][1] + sig[2] * t.g[b][2],
+                       sig[3] * t.g[b][0] + sig[4] * t.g[b][1] + sig[5] * t.g[b][2],
+                       sig[6] * t.g[b][0] + sig[7] * t.g[b][1] + sig[8] * t.g[b][2]};
+#pragma unroll
+      for (int a = 0; a <= b; ++a) s[a][b] = s[b][a] = t.g[a][0] * sg[0] + t.g[a][1] * sg[1] + t.g[a][2] * sg[2];
+    }
+    T* o = out + e * 144;
+#pragma unroll
+    for (int a = 0; a < 4; ++a)
+#pragma unroll
+      for (int i = 0; i < 3; ++i) {
+        T v[12];
+#pragma unroll
+        for (int c = 0; c < 12; ++c) v[c] = (c % 3 == i) ? s[a][c / 3] : T(0);
+        store_row12(o + 12 * (3 * a + i), v);
+      }
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -415,24 +466,33 @@ __global__ void __launch_bounds__(512) solid_K_kernel(const T* __restrict__ coor
 //            K_ab = lam S + mu S^T + mu tr(S) I and its mirror image go to the warp's K tile
 //   store    the tile leaves through the TMA engine while the warp is already in phase A of its next element
 // Connectivity is requested two elements ahead and coordinates one element ahead.
+//
+// GEO = true: the geometric stiffness of the stress of `disp` (femb_solid_geometric) with the same layout.  Displacements are
+// gathered beside the coordinates; in phase A lane (q, h) also forms G = sum_a dN_a (x) u_a, H = J^-1 G and
+// S_q = w_q |detJ_q| sigma_q in registers and stores t_a = S_q g_a next to g_a (ts[q][a][3]); in phase B the tile's lane sums
+// s_ab = sum_q t_a . g_b (6 FMAs per point) and the blocks s_ab I3 go through the same tile and TMA store.
 // ------------------------------------------------------------------------------------------------
 constexpr int C10W_WARPS = 4, C10W_MAXQ = 16;
 constexpr int C10W_GQ = 36;   // gs row stride per point (30 used): with 36 the 128-bit stores of phase A and loads of phase B are conflict-free
 constexpr int C10W_PER_WARP = 900 + C10W_MAXQ * C10W_GQ + C10W_MAXQ + 32;   // K tile | gs | wd | xs   (T units, a multiple of 4)
+constexpr int C10W_PER_WARP_GEO = C10W_PER_WARP + 32 + C10W_MAXQ * C10W_GQ;  // ... | us | ts
 
 // NQ > 0: the number of points is a compile-time constant (the reference's 11-point rule): phase B unrolls completely and its
 // loads run ahead of the FMAs of earlier points; NQ = 0: any nq_rt <= 16.
-template <typename T, typename I, int MINB, int NQ>
+template <typename T, typename I, int MINB, int NQ, bool GEO>
 __global__ void __launch_bounds__(C10W_WARPS * 32, MINB) c3d10_K_warp_kernel(const T* __restrict__ coords, const I* __restrict__ conn, long long M,
-                                                                             SolidTab tab, int nq_rt, T lam, T mu, T* __restrict__ out) {
+                                                                             SolidTab tab, int nq_rt, T lam, T mu, T* __restrict__ out,
+                                                                             const T* __restrict__ disp) {
   constexpr int NEN = 10, ND = 30;
   const int nq = NQ ? NQ : nq_rt;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  T* kt = reinterpret_cast<T*>(smem_raw) + (size_t)w * C10W_PER_WARP;
+  T* kt = reinterpret_cast<T*>(smem_raw) + (size_t)w * (GEO ? C10W_PER_WARP_GEO : C10W_PER_WARP);
   T* gs = kt + ND * ND;
   T* wd = gs + C10W_MAXQ * C10W_GQ;
   T* xs = wd + C10W_MAXQ;
+  T* us = xs + 32;                // GEO only
+  T* ts = us + 32;                // GEO only
   const long long nwarps = (long long)gridDim.x * C10W_WARPS, warp0 = (long long)blockIdx.x * C10W_WARPS + w;
   // phase-A role
   const int q = lane >> 1, h = lane & 1;
@@ -458,13 +518,68 @@ __global__ void __launch_bounds__(C10W_WARPS * 32, MINB) c3d10_K_warp_kernel(con
   T xv = 0;           // coordinate of the current element
   if (warp0 < M) xv = __ldg(coords + 3 * ldidx(conn + warp0 * NEN + ga) + gc);
   if (warp0 + nwarps < M) n1 = ldidx(conn + (warp0 + nwarps) * NEN + ga);
+  T uv = 0;           // GEO: displacement of the current element
+  if (GEO && warp0 < M) uv = __ldg(disp + 3 * ldidx(conn + warp0 * NEN + ga) + gc);
   for (long long e = warp0; e < M; e += nwarps) {
     xs[lane] = xv;
+    if (GEO) us[lane] = uv;
     __syncwarp();
+    if (GEO && e + nwarps < M) uv = __ldg(disp + 3 * n1 + gc);
     if (e + nwarps < M) xv = __ldg(coords + 3 * n1 + gc);
     if (e + 2 * nwarps < M) n1 = ldidx(conn + (e + 2 * nwarps) * NEN + ga);
     // ---- phase A
-    if (act) {
+    if constexpr (GEO) {
+      if (act) {
+        T J[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0}, G[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+#pragma unroll
+        for (int a = 0; a < NEN; ++a)
+#pragma unroll
+          for (int i = 0; i < 3; ++i)
+#pragma unroll
+            for (int k = 0; k < 3; ++k) J[3 * i + k] += dn[a][i] * xs[3 * a + k], G[3 * i + k] += dn[a][i] * us[3 * a + k];
+        T Ji[9], S[9];
+        const T wa = fabs(inv3(J, Ji)) * wq;
+        {
+          T H[9];   // H[i][k] = du_k / dx_i
+#pragma unroll
+          for (int i = 0; i < 3; ++i)
+#pragma unroll
+            for (int k = 0; k < 3; ++k) H[i * 3 + k] = Ji[i * 3] * G[k] + Ji[i * 3 + 1] * G[3 + k] + Ji[i * 3 + 2] * G[6 + k];
+          const T tr = lam * (H[0] + H[4] + H[8]);
+#pragma unroll
+          for (int i = 0; i < 3; ++i)
+#pragma unroll
+            for (int k = 0; k < 3; ++k) S[3 * i + k] = wa * (mu * (H[3 * i + k] + H[3 * k + i]) + (i == k ? tr : T(0)));
+        }
+        T gv[18], tv[18];
+#pragma unroll
+        for (int aa = 0; aa < 6; ++aa) {
+          const int ah = aa < 4 ? aa + 6 : aa;
+          const T d0 = h ? dn[ah][0] : dn[aa][0], d1 = h ? dn[ah][1] : dn[aa][1], d2 = h ? dn[ah][2] : dn[aa][2];
+          const T g0 = Ji[0] * d0 + Ji[1] * d1 + Ji[2] * d2, g1 = Ji[3] * d0 + Ji[4] * d1 + Ji[5] * d2, g2 = Ji[6] * d0 + Ji[7] * d1 + Ji[8] * d2;
+          gv[3 * aa] = g0, gv[3 * aa + 1] = g1, gv[3 * aa + 2] = g2;
+#pragma unroll
+          for (int i = 0; i < 3; ++i) tv[3 * aa + i] = S[3 * i] * g0 + S[3 * i + 1] * g1 + S[3 * i + 2] * g2;
+        }
+        const int nv = h ? 12 : 18;
+        T* g = gs + q * C10W_GQ + h * 18;
+        T* tq = ts + q * C10W_GQ + h * 18;
+        if (sizeof(T) == 8) {
+          double2* g2 = reinterpret_cast<double2*>(g);
+          double2* t2 = reinterpret_cast<double2*>(tq);
+#pragma unroll
+          for (int k = 0; k < 9; ++k)
+            if (2 * k < nv) {
+              g2[k] = make_double2((double)gv[2 * k], (double)gv[2 * k + 1]);
+              t2[k] = make_double2((double)tv[2 * k], (double)tv[2 * k + 1]);
+            }
+        } else {
+#pragma unroll
+          for (int k = 0; k < 18; ++k)
+            if (k < nv) g[k] = gv[k], tq[k] = tv[k];
+        }
+      }
+    } else if (act) {
       T J[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
       T xr[30];
       if (sizeof(T) == 8) {  // the same address for the whole warp: 15 broadcast 128-bit loads
@@ -517,6 +632,30 @@ __global__ void __launch_bounds__(C10W_WARPS * 32, MINB) c3d10_K_warp_kernel(con
     }
     __syncwarp();
     // ---- phase B
+    T k0[9], k1[9];
+    if constexpr (GEO) {
+      T s0 = 0, s1 = 0;
+#pragma unroll
+      for (int p = 0; p < (NQ ? NQ : C10W_MAXQ); ++p) {
+        if (!NQ && p >= nq) break;
+        const T* g = gs + p * C10W_GQ;
+        const T* tq = ts + p * C10W_GQ + 6 * t;
+        T ar[6];
+        if (sizeof(T) == 8) {
+          const double2* v = reinterpret_cast<const double2*>(tq);
+          const double2 v0 = v[0], v1 = v[1], v2 = v[2];
+          ar[0] = (T)v0.x, ar[1] = (T)v0.y, ar[2] = (T)v1.x, ar[3] = (T)v1.y, ar[4] = (T)v2.x, ar[5] = (T)v2.y;
+        } else {
+#pragma unroll
+          for (int k = 0; k < 6; ++k) ar[k] = tq[k];
+        }
+        const T gb0 = g[3 * b], gb1 = g[3 * b + 1], gb2 = g[3 * b + 2];
+        s0 += ar[0] * gb0 + ar[1] * gb1 + ar[2] * gb2;
+        s1 += ar[3] * gb0 + ar[4] * gb1 + ar[5] * gb2;
+      }
+#pragma unroll
+      for (int k = 0; k < 9; ++k) k0[k] = k % 4 ? T(0) : s0, k1[k] = k % 4 ? T(0) : s1;
+    } else {
     T S0[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0}, S1[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
 #pragma unroll
     for (int p = 0; p < (NQ ? NQ : C10W_MAXQ); ++p) {
@@ -540,7 +679,6 @@ __global__ void __launch_bounds__(C10W_WARPS * 32, MINB) c3d10_K_warp_kernel(con
         S1[3 * i] += u1 * gb0, S1[3 * i + 1] += u1 * gb1, S1[3 * i + 2] += u1 * gb2;
       }
     }
-    T k0[9], k1[9];
     {
       const T tr0 = mu * (S0[0] + S0[4] + S0[8]), tr1 = mu * (S1[0] + S1[4] + S1[8]);
 #pragma unroll
@@ -553,6 +691,7 @@ __global__ void __launch_bounds__(C10W_WARPS * 32, MINB) c3d10_K_warp_kernel(con
       // diagonal blocks: one triangle decides both (w g_i g_j and w g_j g_i round differently)
       if (b == a0) k0[3] = k0[1], k0[6] = k0[2], k0[7] = k0[5];
       if (b == a1) k1[3] = k1[1], k1[6] = k1[2], k1[7] = k1[5];
+    }
     }
     // the previous tile must have been read out of shared memory before it is overwritten
     if (lane == 0) bulk_wait_read();
@@ -599,16 +738,17 @@ __global__ void __launch_bounds__(C10W_WARPS * 32, MINB) c3d10_K_warp_kernel(con
   if (lane == 0) bulk_wait_all();
 }
 
-template <typename T, typename I, int MINB, int NQ>
-static int launch_c3d10_warp(const T* X, const I* C, long long M, SolidTab tab, int nq, T lam, T mu, T* O, cudaStream_t s) {
-  const size_t smem = sizeof(T) * (size_t)C10W_WARPS * C10W_PER_WARP;
-  auto kern = c3d10_K_warp_kernel<T, I, MINB, NQ>;
+template <typename T, typename I, int MINB, int NQ, bool GEO = false>
+static int launch_c3d10_warp(const T* X, const I* C, long long M, SolidTab tab, int nq, T lam, T mu, T* O, cudaStream_t s,
+                             const T* D = nullptr) {
+  const size_t smem = sizeof(T) * (size_t)C10W_WARPS * (GEO ? C10W_PER_WARP_GEO : C10W_PER_WARP);
+  auto kern = c3d10_K_warp_kernel<T, I, MINB, NQ, GEO>;
   FEMB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
   FEMB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, C10W_WARPS * 32, smem));
   if (per_sm < 1) per_sm = 1;
   const int grid = (int)std::min<long long>((M + C10W_WARPS - 1) / C10W_WARPS, (long long)SMS * per_sm);
-  kern<<<grid, C10W_WARPS * 32, smem, s>>>(X, C, M, tab, nq, lam, mu, O);
+  kern<<<grid, C10W_WARPS * 32, smem, s>>>(X, C, M, tab, nq, lam, mu, O, D);
   FEMB_LAUNCH_CHECK();
   return FEMB_OK;
 }
@@ -917,6 +1057,28 @@ static int stress_dispatch(const void* coords, const void* conn, long long M, co
   return FEMB_OK;
 }
 
+template <typename T, typename I>
+static int geometric_dispatch(int kind, const void* coords, const void* conn, long long M, const void* disp, const double* pts, int nq,
+                              double E, double nu, void* out, cudaStream_t s) {
+  if (M == 0) return FEMB_OK;
+  const double c = E / ((1 + nu) * (1 - 2 * nu));
+  const T lam = (T)(c * nu), mu = (T)(c * (1 - 2 * nu) / 2);
+  const T* X = static_cast<const T*>(coords);
+  const I* C = static_cast<const I*>(conn);
+  const T* D = static_cast<const T*>(disp);
+  T* O = static_cast<T*>(out);
+  if (kind == FEMB_C3D4) {
+    c3d4_geometric_kernel<T, I><<<grid_for(M, 128), 128, 0, s>>>(X, C, M, D, lam, mu, O);
+    FEMB_LAUNCH_CHECK();
+    return FEMB_OK;
+  }
+  Scratch scr(s);
+  SolidTab tab;
+  if (int rc = upload_tables<10>(pts, nq, scr, s, tab)) return rc;
+  if (nq == 14) return launch_c3d10_warp<T, I, 3, 14, true>(X, C, M, tab, nq, lam, mu, O, s, D);   // the default degree-5 rule
+  return launch_c3d10_warp<T, I, 3, 0, true>(X, C, M, tab, nq, lam, mu, O, s, D);
+}
+
 template <typename I>
 __global__ void to_c3d4_kernel(const I* __restrict__ conn, long long M, int nen, int k, const int* __restrict__ table, long long* __restrict__ out) {
   const long long total = M * k * 4;
@@ -1008,6 +1170,17 @@ extern "C" int femb_solid(int kind, int what, const void* coords, int fp, const 
   FEMB_CHECK_ARG((fp == 4 || fp == 8) && (ib == 4 || ib == 8), "fp in {4,8}, ib in {4,8}");
   FEMB_CHECK_ARG(pts_host != nullptr, "pts_host");
   return DISPATCH_TI(solid_dispatch_kind, fp, ib, kind, what, coords, conn, M, pts_host, nq, E, nu, out, as_stream(stream));
+}
+
+extern "C" int femb_solid_geometric(int kind, const void* coords, int fp, const void* conn, int ib, int64_t M, const void* disp,
+                                    const double* pts_host, int nq, double E, double nu, void* out, femb_stream stream) {
+  FEMB_CHECK_ARG((fp == 4 || fp == 8) && (ib == 4 || ib == 8), "fp in {4,8}, ib in {4,8}");
+  FEMB_CHECK_ARG(kind == FEMB_C3D4 || kind == FEMB_C3D10, "femb_solid_geometric: kind must be C3D4 or C3D10");
+  FEMB_CHECK_ARG(M >= 0, "M >= 0");
+  FEMB_CHECK_ARG(kind == FEMB_C3D4 || (pts_host != nullptr && nq >= 1 && nq <= C10W_MAXQ),
+                 "femb_solid_geometric: C3D10 needs pts_host [nq,4] with 1 <= nq <= 16");
+  FEMB_CHECK_ARG(M == 0 || (coords && conn && disp && out), "femb_solid_geometric: coords, conn, disp and out must be non-null");
+  return DISPATCH_TI(geometric_dispatch, fp, ib, kind, coords, conn, M, disp, pts_host, nq, E, nu, out, as_stream(stream));
 }
 
 extern "C" int femb_default_points(int kind, double* p) {

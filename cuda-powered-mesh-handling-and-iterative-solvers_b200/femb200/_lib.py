@@ -31,6 +31,7 @@ SIGNATURES = {
     "femb_default_points": [c_i32, C.POINTER(c_f64)],
     "femb_mass_points": [c_i32, C.POINTER(c_f64)],
     "femb_solid_stress": [c_i32, c_vp, c_i32, c_vp, c_i32, c_i64, c_vp, C.POINTER(c_f64), c_i32, c_f64, c_f64, c_i32, c_vp, c_vp, c_vp],
+    "femb_solid_geometric": [c_i32, c_vp, c_i32, c_vp, c_i32, c_i64, c_vp, C.POINTER(c_f64), c_i32, c_f64, c_f64, c_vp, c_vp],
     "femb_shape_tables": [c_i32, C.POINTER(c_f64), c_i32, C.POINTER(c_f64), C.POINTER(c_f64)],
     "femb_stress_helper": [c_i32, c_vp, c_i32, c_i64, c_vp, c_vp],
     "femb_node_average": [c_vp, c_vp, c_i32, c_vp, c_vp],

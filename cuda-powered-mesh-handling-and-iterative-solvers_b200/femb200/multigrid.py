@@ -49,10 +49,11 @@ class Level:
         self.n = 3 * self.nodes
         plan = self.plan = ops.CsrPlan(tets, self.nodes, dev)
         brow, bcol = plan.pattern(1)
+        keep_m = keep_km and rho is not None   # rho None: K alone (buckling needs no mass)
         Ke = element_module.compute_c3d4_K_matrix(coords, tets, E, nu, device=dev, dtype=torch.float64)
-        Me = element_module.compute_c3d4_M_matrix(coords, tets, rho, device=dev, dtype=torch.float64) if (shift or keep_km) else None
+        Me = element_module.compute_c3d4_M_matrix(coords, tets, rho, device=dev, dtype=torch.float64) if (shift or keep_m) else None
         self.K = ops.Bsr3.from_csr_values(brow, bcol, plan.assemble(Ke, 3)) if (keep_km or not shift) else None
-        self.M = ops.Bsr3.from_csr_values(brow, bcol, plan.assemble(Me, 3)) if keep_km else None
+        self.M = ops.Bsr3.from_csr_values(brow, bcol, plan.assemble(Me, 3)) if keep_m else None
         self.A = self.K if not shift else ops.Bsr3.from_csr_values(brow, bcol, plan.assemble(Ke + shift * Me, 3))
         del Ke, Me
         self.mask = dof_mask(self.nodes, fixed_fn(coords), dev)
@@ -68,7 +69,8 @@ class Level:
 
 class Hierarchy:
     """Coarse C3D4 mesh (coords, tets) + `levels` uniform refinements with their operators and the coarse factor.  `fixed_fn(coords_l)`
-    gives the clamped node ids of every level.  `self.L[-1]` is the finest level; its K and M (shift-free) are kept for LOBPCG."""
+    gives the clamped node ids of every level.  `self.L[-1]` is the finest level; its K and M (shift-free) are kept for LOBPCG
+    (rho = None with shift = 0: no mass is assembled, the finest level keeps K only)."""
 
     def __init__(self, coords, tets, levels, fixed_fn, E, nu, rho, shift, dev, element_module):
         self.dev, self.shift = dev, float(shift)
@@ -163,11 +165,12 @@ class Hierarchy:
 
 
 class MultilevelBackend(modes.DeviceBackend):
-    """LOBPCG backend whose residual step preconditions with the V-cycle instead of Jacobi.  K, M, mask: those of the finest level."""
+    """LOBPCG backend whose residual step preconditions with the V-cycle instead of Jacobi.  The pencil (A, B) defaults to the finest
+    level's (K, M); mask: the finest level's."""
 
-    def __init__(self, H):
+    def __init__(self, H, A=None, B=None):
         top = H.L[-1]
-        super().__init__(top.K, top.M, top.mask)
+        super().__init__(top.K if A is None else A, top.M if B is None else B, top.mask)
         self.H = H
         self.maskf = top.mask.to(torch.float64)
 

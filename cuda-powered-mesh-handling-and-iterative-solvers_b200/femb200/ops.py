@@ -152,6 +152,25 @@ def solid_stress(kind, coords, elements, displacement, points, E, nu, single=Tru
     return S, V
 
 
+def solid_geometric(kind, coords, elements, displacement, points, E, nu, device="cuda:0", dtype=torch.float32):
+    """Geometric stiffness [M, 3nen, 3nen] of the stress of `displacement` (kind C3D4 or C3D10; points: [xi,eta,zeta,w] rows,
+    ignored for C3D4).  The displacement is cast to `dtype`."""
+    dev = cuda_device(device)
+    x, conn, u = real(coords, dev, dtype), index(elements, dev), real(displacement, dev, dtype)
+    nen = _NEN[kind]
+    if conn.shape[1] != nen:
+        raise ValueError(f"elements must be [M,{nen}] for this element type, got {tuple(conn.shape)}")
+    if u.shape != x.shape:
+        raise ValueError(f"displacement must be [N,3] like coords, got {tuple(u.shape)} vs {tuple(x.shape)}")
+    M, nd = conn.shape[0], 3 * nen
+    out = torch.empty((M, nd, nd), device=dev, dtype=dtype)
+    flat = [v for row in points for v in row]
+    with torch.cuda.device(dev):
+        check(lib.femb_solid_geometric(kind, _p(x), _fp(x), _p(conn), _fp(conn), M, _p(u), _host_doubles(flat), len(points), float(E),
+                                       float(nu), _p(out), _stream(dev)), "femb_solid_geometric")
+    return out
+
+
 def stress_helper(what, t):
     """what 0: Voigt [M,6] -> [M,3,3]; 1: [M,3,3] -> von Mises [M].  Works on the tensor's own device/dtype like the reference."""
     t = torch.as_tensor(t)

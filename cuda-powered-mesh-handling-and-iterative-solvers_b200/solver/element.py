@@ -269,6 +269,12 @@ def compute_c3d4_element_stress(coords, elements, displacement, E, nu, device="c
     return _ops.solid_stress(_ops.C3D4, coords, elements, displacement, [[0.25, 0.25, 0.25, 1.0]], E, nu, True, device, dtype)
 
 
+def compute_c3d4_KG_matrix(coords, elements, displacement, E, nu, device="cuda:0", dtype=torch.float32):
+    """Geometric stiffness [M,12,12] of the constant stress of `displacement` [N,3]: block (a,b) = V g_a^T sigma g_b I3.
+    Not in the reference (parity unpinned); the initial-stress matrix of linear buckling (solver.buckling_modes)."""
+    return _ops.solid_geometric(_ops.C3D4, coords, elements, displacement, [[0.25, 0.25, 0.25, 1.0]], E, nu, device, dtype)
+
+
 def c3d10_to_c3d4(c3d10_elements, device="cuda:0"):
     """8 children per C3D10 (element.py:963-993)."""
     return _ops.to_c3d4(_ops.C3D10, c3d10_elements, device)
@@ -293,12 +299,16 @@ def _solid_K(kind, coords, elements, E, nu, integral_point, single, device, dtyp
     return _solid(kind, 3 if single else 4, coords, elements, integral_point, device, dtype, E, nu, single_point=False, out=out)
 
 
-def _solid_M(kind, coords, elements, rho, integral_point, device, dtype):
+def _exact_pts(kind, integral_point, dtype):
+    """The rule of the operators that are not in the reference (mass, geometric stiffness): the caller's points, or by default
+    femb_mass_points (for C3D10 the degree-5 14-point rule, not the reference's 11-point rule whose weights sum to 0.45)."""
     if integral_point is None:
-        pts = torch.tensor(_ops.mass_points(kind), dtype=torch.float64).to(dtype).to(torch.float64).tolist()
-    else:
-        pts = _pts(kind, integral_point, dtype)
-    return _ops.solid(kind, 6, coords, elements, pts, rho, 0.0, device, dtype)
+        return torch.tensor(_ops.mass_points(kind), dtype=torch.float64).to(dtype).to(torch.float64).tolist()
+    return _pts(kind, integral_point, dtype)
+
+
+def _solid_M(kind, coords, elements, rho, integral_point, device, dtype):
+    return _ops.solid(kind, 6, coords, elements, _exact_pts(kind, integral_point, dtype), rho, 0.0, device, dtype)
 
 
 def compute_c3d10_Jacobian(coords, elements, integral_point, device="cuda:0", dtype=torch.float32):
@@ -327,6 +337,14 @@ def compute_c3d10_element_stress(coords, elements, displacement, E, nu, integral
     """single=True: ([M,3,3],[M]) weighted with the rule's weights (which sum to 0.45, q4); single=False:
     ([n_int,M,3,3],[n_int,M]) (element.py:1127-1189)."""
     return _stress(_ops.C3D10, coords, elements, displacement, E, nu, integral_point, single, device, dtype, True)
+
+
+def compute_c3d10_KG_matrix(coords, elements, displacement, E, nu, integral_point=None, device="cuda:0", dtype=torch.float32):
+    """Geometric stiffness sum_q w_q |detJ_q| g_a^T sigma_q g_b I3, [M,30,30], of the stress of `displacement` [N,3]; default
+    rule = degree-5 14-point (exact for straight-sided tets), integral_point [nq<=16, 4] rows (xi, eta, zeta, w) otherwise.
+    Not in the reference -- parity unpinned."""
+    return _ops.solid_geometric(_ops.C3D10, coords, elements, displacement, _exact_pts(_ops.C3D10, integral_point, dtype), E, nu,
+                                device, dtype)
 
 
 def compute_c3d10_M_matrix(coords, elements, rho, integral_point=None, device="cuda:0", dtype=torch.float32):

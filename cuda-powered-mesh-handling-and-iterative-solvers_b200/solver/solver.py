@@ -590,6 +590,102 @@ def subdivided_lowest_modes(coords, elements, levels, fixed_fn, E, nu, rho, num_
     return out + (info,) if return_info else out
 
 
+def _buckling_args(num_eigs, fixed_nodes):
+    if not 1 <= num_eigs <= 12:
+        raise ValueError("num_eigs must be between 1 and 12")
+    f = torch.as_tensor(fixed_nodes if fixed_nodes is not None else [])
+    if f.numel() == 0 or (f.dtype == torch.bool and not bool(f.any())):
+        raise ValueError("no node is fixed: a free-free model has no linear buckling problem (K is singular)")
+
+
+def _buckling_report(kind, info, max_iter):
+    if info["status"] == "converged":
+        print(f"{kind} buckling LOBPCG converged after {info['iterations']} iterations (reference solve: {info['static_iterations']} iterations).")
+    else:
+        print(f"{kind} buckling LOBPCG did not converge within {max_iter} iterations; max residual {info['residuals'].max():.3e}.")
+
+
+def buckling_modes(coords, elements, F, fixed, E, nu, num_eigs=4, tol=1e-8, max_iter=2000, static_tol=1e-10, static_max_iter=20000,
+                   integral_point=None, device="cuda:0", dtype=torch.float64, return_info=False, verbose=True):
+    """Linear buckling of a C3D4 (elements [M,4]) or C3D10 ([M,10]) mesh under the reference load F [N,3] (not in the reference).
+    The reference state u_ref = K^-1 F comes from the device Jacobi-PCG (|F - K u| <= static_tol |F|, else ValueError), K_G is the
+    geometric stiffness of its stress, and LOBPCG with the Jacobi preconditioner of K solves K_G phi = nu K phi on the free dofs
+    (femb200/buckling.py).  Load factor lam = -1/nu for nu < 0, +inf for nu >= 0 (no buckling in that pair): (K + lam K_G) phi = 0.
+    `fixed`: node ids or a bool node mask, all three dofs clamped (a free-free model is refused).  C3D10 integrates K and K_G with
+    `integral_point` [nq<=16, 4] rows (xi, eta, zeta, w), by default the degree-5 14-point rule (exact for straight-sided tets), not
+    the reference's 11-point rule; like compute_c3d10_K_matrix it needs detJ > 0.  1 <= num_eigs <= 12; a pair has converged when |K_G x - nu K x| / ((|K_G|_1 + |nu| |K|_1) |x|)
+    <= tol (max_iter reached: status "maxiter", no error).  A repeated call returns bit-identical results.
+    Returns (load_factors [num_eigs] ascending, modes [3N, num_eigs] K-orthonormal with zeros on fixed dofs, u_ref [N,3]) cast to
+    `dtype`; with return_info also the dict of lowest_modes without freq_hz, plus nu (the pencil's eigenvalues) and
+    static_iterations / static_residual of the reference solve."""
+    from femb200 import buckling
+    dev = _ops.cuda_device(device)
+    elements = _ops.index(elements, dev)
+    if elements.dim() != 2 or elements.shape[1] not in (4, 10):
+        raise ValueError(f"elements must be [M,4] (C3D4) or [M,10] (C3D10), got {tuple(elements.shape)}")
+    _buckling_args(num_eigs, fixed)
+    coords = _ops.real(coords, dev, torch.float64)
+    N = coords.shape[0]
+    mask = _dof_mask(N, 3, fixed, dev)
+    plan = _ops.CsrPlan(elements, N, dev)
+    brow, bcol = plan.pattern(1)
+    if elements.shape[1] == 4:
+        Ke = _el.compute_c3d4_K_matrix(coords, elements, E, nu, device=dev, dtype=torch.float64)
+    else:
+        rule = torch.tensor(_el._exact_pts(_ops.C3D10, integral_point, torch.float64), dtype=torch.float64)
+        Ke = _el.compute_c3d10_K_matrix(coords, elements, E, nu, integral_point=rule, device=dev, dtype=torch.float64)
+    K = _ops.Bsr3.from_csr_values(brow, bcol, plan.assemble(Ke, 3))
+    del Ke
+    u, static_its, static_res = buckling.static_jacobi(K, mask, F, static_tol, static_max_iter)
+    u = u.reshape(N, 3)
+    if elements.shape[1] == 4:
+        KGe = _el.compute_c3d4_KG_matrix(coords, elements, u, E, nu, device=dev, dtype=torch.float64)
+    else:
+        KGe = _el.compute_c3d10_KG_matrix(coords, elements, u, E, nu, integral_point=rule, device=dev, dtype=torch.float64)
+    KG = _ops.Bsr3.from_csr_values(brow, bcol, plan.assemble(KGe, 3))
+    del KGe
+    lam, modes_out, info = buckling.solve(buckling.JacobiBackend(KG, K, mask), num_eigs, tol, max_iter)
+    info["static_iterations"], info["static_residual"] = static_its, static_res
+    if verbose:
+        _buckling_report("Jacobi", info, max_iter)
+    out = (torch.from_numpy(lam).to(device=dev, dtype=dtype), modes_out.contiguous().to(dtype), u.to(dtype))
+    return out + (info,) if return_info else out
+
+
+def subdivided_buckling_modes(coords, elements, levels, load_fn, fixed_fn, E, nu, num_eigs=4, tol=1e-8, max_iter=500, static_tol=1e-10,
+                              static_max_iter=500, device="cuda:0", dtype=torch.float64, return_info=False, verbose=True):
+    """Linear buckling on a refined C3D4 mesh (not in the reference): the coarse mesh (coords, elements [M,4]) is refined `levels` times
+    as in subdivided_lowest_modes, load_fn(coords_l, tets_l) -> F [N_l, 3] gives the reference load on the finest mesh and
+    fixed_fn(coords_l) the clamped node ids on every level.  What buckling_modes computes on the finest mesh, with the Jacobi
+    preconditioner replaced by one V-cycle over the hierarchy (femb200/multigrid.py at shift 0) in both the reference solve (PCG) and
+    LOBPCG, so the iteration counts stay roughly flat as the mesh is refined.  No mass is assembled.  The coarse mesh may hold at most
+    multigrid.MAX_COARSE_DOFS free dofs.  Returns (load_factors, modes, u_ref, coords_fine, elements_fine) (+ info, which also holds
+    `levels`: nodes, tets, dofs per level, coarsest first)."""
+    from femb200 import buckling, multigrid
+    dev = _ops.cuda_device(device)
+    elements = _ops.index(elements, dev)
+    if elements.dim() != 2 or elements.shape[1] != 4:
+        raise ValueError(f"subdivided_buckling_modes refines C3D4 meshes: elements must be [M,4], got {tuple(elements.shape)}")
+    if int(levels) != levels or levels < 0:
+        raise ValueError("levels must be a non-negative integer")
+    coords = _ops.real(coords, dev, torch.float64)
+    _buckling_args(num_eigs, fixed_fn(coords))
+    H = multigrid.Hierarchy(coords, elements, int(levels), fixed_fn, E, nu, None, 0.0, dev, _el)
+    top = H.L[-1]
+    u, static_its, static_res = buckling.static_multigrid(H, load_fn(H.coords, H.tets), static_tol, static_max_iter)
+    u = u.reshape(-1, 3)
+    KGe = _el.compute_c3d4_KG_matrix(H.coords, H.tets, u, E, nu, device=dev, dtype=torch.float64)
+    brow, bcol = top.plan.pattern(1)
+    KG = _ops.Bsr3.from_csr_values(brow, bcol, top.plan.assemble(KGe, 3))
+    del KGe
+    lam, modes_out, info = buckling.solve(buckling.MultilevelBackend(H, KG), num_eigs, tol, max_iter)
+    info["static_iterations"], info["static_residual"], info["levels"] = static_its, static_res, H.describe()
+    if verbose:
+        _buckling_report("Multigrid", info, max_iter)
+    out = (torch.from_numpy(lam).to(device=dev, dtype=dtype), modes_out.contiguous().to(dtype), u.to(dtype), H.coords, H.tets)
+    return out + (info,) if return_info else out
+
+
 def static_structure_solver(coords, force, fixed, c3d4=None, c3d6=None, c3d8=None, s3=None, s4=None, material=None, u_init=None,
                             tol=1e-10, max_iter=1000, device="cuda:0", dtype=torch.float64, eps=1e-30, return_info=False, verbose=True):
     """Mixed-element static solve on [N,6] (solver.py:11-135): solids act on the translations, shells on all six dofs

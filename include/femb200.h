@@ -94,6 +94,13 @@ int femb_solid_stress(int kind, const void* coords, int fp, const void* conn, in
                       const double* pts_host, int nq, double E, double nu, int single, void* stress, void* vm,
                       femb_stream stream);
 
+/* Geometric stiffness of the stress state of a displacement field (not in the reference).
+ * kind = FEMB_C3D4 (one point, pts ignored) or FEMB_C3D10 (pts_host [nq,4] on the host, 1 <= nq <= 16; other kinds -> error).
+ * disp [N,3] in the precision of coords.  At every point q: eps = sym(sum_c u_c (x) g_c), sigma = lam tr(eps) I + 2 mu eps,
+ * s_ab = sum_q w_q |detJ_q| g_a^T sigma_q g_b;  out [M, 3nen, 3nen] with block (a,b) = s_ab I3 (bitwise symmetric). */
+int femb_solid_geometric(int kind, const void* coords, int fp, const void* conn, int ib, int64_t M, const void* disp,
+                         const double* pts_host, int nq, double E, double nu, void* out, femb_stream stream);
+
 /* Shell elements (solver/shell.py): compute_s3_* :297-453, compute_s4_* :597-861.
  * what = 0: unit [M,3,3]; 1: J [M,2,2]; 2: gradients [M,nen,2]; 3: B [M,6,6nen]; 4: K [M,6nen,6nen];
  *        5: (S4) per-point K [M,24,24,nq] (single=False).  S3 ignores pts. D6 = Kirchhoff D as 36 doubles (host). */
