@@ -14,6 +14,8 @@
 //   mg_smooth        one damped-Jacobi step X_out = X_in + omega dinv (R - A X_in) and/or the residual R - A X_in, on the SpMM's
 //                    block traversal (each 3x3 block of A read once for all m columns)
 //   mg_transfer      Y (+)= mask (S (x) I3) X for a node-level scalar CSR S: the prolongation P and the restriction R = P^T
+// and one to the smoothed-aggregation hierarchy of femb200/amg.py, whose transfers are rectangular 3x3 block-CSR matrices:
+//   mg_transfer_bsr3 Y (+)= mask (T X) on the SpMM's block traversal
 #include "common.cuh"
 #include "spmv_dev.cuh"
 
@@ -295,6 +297,25 @@ __global__ void __launch_bounds__(MB_THREADS) mg_transfer_kernel(long long n_out
   }
 }
 
+// Y (+)= mask_out (T X) for a rectangular 3x3 block-CSR T (n_out block rows, columns < n_in): the SpMM's traversal with an
+// epilogue that masks and writes or accumulates.
+__global__ void __launch_bounds__(MB_THREADS) mg_transfer_bsr3_kernel(long long n_out, const int* __restrict__ trow, const int* __restrict__ tcol,
+                                                                       const double* __restrict__ tval, const unsigned char* __restrict__ mask_out,
+                                                                       int m, int log_mp, const double* __restrict__ X, long long ldx, int accumulate,
+                                                                       double* __restrict__ Y, long long ldy) {
+  bsr3_warp_rows<false>(n_out, trow, tcol, tval, nullptr, nullptr, m, log_mp, X, ldx,
+                        [&](long long row, int c, double t0, double t1, double t2, double, double, double) {
+                          const double t[3] = {t0, t1, t2};
+#pragma unroll
+                          for (int d = 0; d < 3; ++d) {
+                            const long long r = 3 * row + d;
+                            const double v = (!mask_out || mask_out[r]) ? t[d] : 0.0;
+                            double* y = Y + r * ldy + c;
+                            *y = accumulate ? *y + v : v;
+                          }
+                        });
+}
+
 // Do the strided views (p, ld_p, kp columns) and (q, ld_q, kq columns) over n rows share an element?  Views with the same leading
 // dimension may interleave (disjoint column windows of one buffer); otherwise any overlap of the address ranges counts.
 static bool spans_meet(const double* p, long long np, const double* q, long long nq) {  // [p, p+np) and [q, q+nq), in doubles
@@ -444,6 +465,24 @@ extern "C" int femb_mg_transfer(int64_t n_out, int64_t n_in, int64_t nnz, const 
   while ((1 << log_mp) < m) ++log_mp;
   mg_transfer_kernel<<<grid_for(n_out * 32, MB_THREADS, 32), MB_THREADS, 0, as_stream(stream)>>>(n_out, crow, col, val, mask_out, m, log_mp, X, ldx,
                                                                                                 accumulate, Y, ldy);
+  FEMB_LAUNCH_CHECK();
+  return FEMB_OK;
+}
+
+extern "C" int femb_mg_transfer_bsr3(int64_t n_out, int64_t n_in, int64_t nnzb, const int32_t* trow, const int32_t* tcol, const double* tval,
+                                     const uint8_t* mask_out, int m, const double* X, int64_t ldx, int accumulate, double* Y, int64_t ldy,
+                                     femb_stream stream) {
+  FEMB_CHECK_ARG(m >= 1 && m <= MB_MAXM, "1 <= m <= 16");
+  FEMB_CHECK_ARG(n_out >= 0 && n_in >= 0 && nnzb >= 0 && nnzb <= INT32_MAX, "n_out, n_in >= 0, 0 <= nnzb < 2^31");
+  FEMB_CHECK_ARG(trow && tcol && tval && X && Y, "non-null trow, tcol, tval, X, Y");
+  FEMB_CHECK_ARG(ldx >= m && ldy >= m, "ldx, ldy >= m");
+  FEMB_CHECK_ARG(accumulate == 0 || accumulate == 1, "accumulate is 0 or 1");
+  FEMB_CHECK_ARG(n_in == 0 || n_out == 0 || !spans_meet(Y, (3 * n_out - 1) * ldy + m, X, (3 * n_in - 1) * ldx + m), "Y overlaps X");
+  if (n_out == 0) return FEMB_OK;
+  int log_mp = 0;
+  while ((1 << log_mp) < m) ++log_mp;
+  mg_transfer_bsr3_kernel<<<grid_for(n_out * 32, MB_THREADS, 32), MB_THREADS, 0, as_stream(stream)>>>(n_out, trow, tcol, tval, mask_out, m, log_mp,
+                                                                                                      X, ldx, accumulate, Y, ldy);
   FEMB_LAUNCH_CHECK();
   return FEMB_OK;
 }

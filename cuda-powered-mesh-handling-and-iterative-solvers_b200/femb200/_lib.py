@@ -87,6 +87,11 @@ SIGNATURES = {
     "femb_lobpcg_residual": [c_i64, c_i32, c_vp, c_i64, c_vp, c_vp, c_i64, C.POINTER(c_f64), c_vp, c_i32, c_vp, c_vp, c_i64, c_vp, c_vp],
     "femb_mg_smooth_bsr3": [c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_f64, c_i32, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp],
     "femb_mg_transfer": [c_i64, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_i64, c_i32, c_vp, c_i64, c_vp],
+    "femb_mg_transfer_bsr3": [c_i64, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_i64, c_i32, c_vp, c_i64, c_vp],
+    "femb_amg_aggregate": [c_i64, c_vp, c_vp, c_vp, c_vp, C.POINTER(c_i64), c_vp],
+    "femb_amg_tentative": [c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_f64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp],
+    "femb_bsr3_spgemm": [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, C.POINTER(c_i64), c_vp],
+    "femb_bsr3_transpose": [c_i64, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp],
     "femb_csr_jacobi": [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp],
     "femb_graph_from_pairs": [c_vp, c_i64, c_i32, c_i64, c_vp, c_vp, c_vp],
     "femb_subdomain_forces": [c_vp, c_i32, c_i64, c_i32, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp],

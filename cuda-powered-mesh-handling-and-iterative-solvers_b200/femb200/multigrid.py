@@ -63,13 +63,43 @@ class Level:
             nc = self.nodes - parents.shape[0]
             self.P = hybrid._prolongation_csr(parents, nc, dev)
             self.R = hybrid._restriction_csr(parents, nc, dev)
-        z = lambda: torch.zeros((self.n, WIDTH), device=dev, dtype=torch.float64)  # noqa: E731
-        self.b, self.x, self.y, self.t = z(), z(), z(), z()
+        self.b, self.x, self.y, self.t = (level_buffer(self.n, dev) for _ in range(4))
+
+    def restrict(self, coarse, na, X, stream):
+        """coarse.b[:, :na] = coarse.mask (R X) (femb_mg_transfer)."""
+        _node_transfer(self.R, coarse.nodes, self.nodes, coarse.mask, na, X, coarse.b, False, stream)
+
+    def prolong(self, coarse, na, Xc, Y, stream):
+        """Y[:, :na] += mask (P Xc) (femb_mg_transfer)."""
+        _node_transfer(self.P, self.nodes, coarse.nodes, self.mask, na, Xc, Y, True, stream)
+
+
+def level_buffer(n, dev):
+    return torch.zeros((n, WIDTH), device=dev, dtype=torch.float64)
+
+
+def _node_transfer(S, n_out, n_in, mask_out, na, X, Y, accumulate, stream):
+    crow, col, val = S
+    with torch.cuda.device(X.device):
+        check(lib.femb_mg_transfer(n_out, n_in, col.numel(), _p(crow), _p(col), _p(val), _p(mask_out), na, _p(X), WIDTH, int(accumulate),
+                                   _p(Y), WIDTH, stream), "femb_mg_transfer")
+
+
+def dense_free_block(A, mask):
+    """(free dof ids, dense A[free][:, free]) of a 3x3 block-CSR operator."""
+    rows = torch.repeat_interleave(torch.arange(A.nb, device=A.dev), (A.brow[1:] - A.brow[:-1]).long())
+    D = torch.zeros((3 * A.nb, 3 * A.nb), device=A.dev, dtype=torch.float64)
+    d = torch.arange(3, device=A.dev)
+    D[(3 * rows[:, None, None] + d[:, None]), (3 * A.bcol.long()[:, None, None] + d[None, :])] = A.bval
+    idx = torch.nonzero(mask).reshape(-1)
+    return idx, D[idx][:, idx]
 
 
 class Hierarchy:
-    """Coarse C3D4 mesh (coords, tets) + `levels` uniform refinements with their operators and the coarse factor.  `fixed_fn(coords_l)`
-    gives the clamped node ids of every level.  `self.L[-1]` is the finest level; its K and M (shift-free) are kept for LOBPCG
+    """V-cycle over levels L[0] (coarsest, dense Cholesky) .. L[-1] (finest).  A level holds A (ops.Bsr3), mask, dinv, nodes, n, the
+    buffers b, x, y, t and, above level 0, restrict / prolong to the level below (femb200/amg.py builds such levels algebraically).
+    Here they come from a coarse C3D4 mesh (coords, tets) + `levels` uniform refinements; `fixed_fn(coords_l)` gives the clamped
+    node ids of every level.  `self.L[-1]` is the finest level; its K and M (shift-free) are kept for LOBPCG
     (rho = None with shift = 0: no mass is assembled, the finest level keeps K only)."""
 
     def __init__(self, coords, tets, levels, fixed_fn, E, nu, rho, shift, dev, element_module):
@@ -89,12 +119,10 @@ class Hierarchy:
         self.stream = torch.cuda.current_stream(dev).cuda_stream
 
     def _factor(self, l0):
-        idx = torch.nonzero(l0.mask).reshape(-1)
-        nf = idx.numel()
+        nf = int(l0.mask.sum())
         if nf > MAX_COARSE_DOFS:
             raise ValueError(f"the coarse mesh has {nf} free dofs; its dense factor allows at most {MAX_COARSE_DOFS}: refine a coarser mesh more often")
-        crow, col = l0.plan.pattern(3)
-        A0 = torch.sparse_csr_tensor(crow, col, l0.A.to_csr_values(), size=(l0.n, l0.n)).to_dense()[idx][:, idx]
+        idx, A0 = dense_free_block(l0.A, l0.mask)
         L, info = torch.linalg.cholesky_ex(A0)
         d = torch.diagonal(L)
         if int(info) != 0 or nf and float((d * d).min()) < SINGULAR_PIVOT * float(torch.diagonal(A0).max()):
@@ -114,12 +142,6 @@ class Hierarchy:
             check(lib.femb_mg_smooth_bsr3(A.nb, A.nnzb, _p(A.brow), _p(A.bcol), _p(A.bval), _p(lv.mask), _p(lv.dinv), OMEGA, na,
                                           _p(lv.b), WIDTH, _p(X_in), WIDTH, _p(X_out, out_c0), X_out.shape[1] if X_out is not None else 0,
                                           _p(res), WIDTH, self.stream), "femb_mg_smooth_bsr3")
-
-    def transfer(self, S, n_out, n_in, mask_out, na, X, Y, accumulate):
-        crow, col, val = S
-        with torch.cuda.device(self.dev):
-            check(lib.femb_mg_transfer(n_out, n_in, col.numel(), _p(crow), _p(col), _p(val), _p(mask_out), na, _p(X), WIDTH, int(accumulate),
-                                       _p(Y), WIDTH, self.stream), "femb_mg_transfer")
 
     def coarse_solve(self):
         """L[0].x = A_0^-1 L[0].b on the free dofs (all WIDTH columns: a fixed shape keeps the library's path, and the result, fixed)."""
@@ -143,9 +165,9 @@ class Hierarchy:
             self.smooth(lv, na, x, y)
             x, y = y, x
         self.smooth(lv, na, x, None, res=lv.t)
-        self.transfer(lv.R, cl.nodes, lv.nodes, cl.mask, na, lv.t, cl.b, False)
+        lv.restrict(cl, na, lv.t, self.stream)
         xc = self.cycle(l - 1, na)
-        self.transfer(lv.P, lv.nodes, cl.nodes, lv.mask, na, xc, x, True)
+        lv.prolong(cl, na, xc, x, self.stream)
         for s in range(SMOOTH):
             if s == SMOOTH - 1 and out is not None:
                 self.smooth(lv, na, x, out, c0)

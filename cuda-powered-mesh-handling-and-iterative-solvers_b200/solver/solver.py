@@ -686,6 +686,85 @@ def subdivided_buckling_modes(coords, elements, levels, load_fn, fixed_fn, E, nu
     return out + (info,) if return_info else out
 
 
+def amg_lowest_modes(coords, K_local, M_local, elements, fixed, num_eigs=6, tol=1e-8, max_iter=500, shift=0.0, device="cuda:0",
+                     dtype=torch.float64, return_info=False, verbose=True):
+    """Lowest eigenpairs of K x = lam M x for any 3-dof solid mesh (not in the reference), as lowest_modes computes them, with LOBPCG
+    preconditioned by one V-cycle of smoothed-aggregation algebraic multigrid (femb200/amg.py) instead of Jacobi: the hierarchy is
+    built on the device from the assembled operator and the node coordinates [N, 3], so no mesh hierarchy is needed and the
+    iteration count stays roughly flat as the mesh is refined.  K_local, M_local, elements, fixed: as lowest_modes (K and M are
+    assembled on one plan).  `shift` >= 0: the cycle approximates (K + shift M)^-1; a free-free model needs shift > 0 (a ValueError
+    says so).  Returns what lowest_modes returns; info also holds `levels` (nodes, dofs, free dofs, nnzb per level, coarsest first),
+    `operator_complexity` and `setup_ms` (aggregation, tentative, lambda, spgemm, factor)."""
+    from femb200 import amg, modes, multigrid
+    dev = _ops.cuda_device(device)
+    if not 1 <= num_eigs <= 12:
+        raise ValueError("num_eigs must be between 1 and 12")
+    if not shift >= 0.0:
+        raise ValueError("shift must be >= 0")
+    coords = _ops.real(coords, dev, torch.float64)
+    N = coords.shape[0]
+    plan = _ops.cached_plan(elements, N, dev)
+    brow, bcol = plan.pattern(1)
+    K = _ops.Bsr3.from_csr_values(brow, bcol, plan.assemble(K_local, 3))
+    M = _ops.Bsr3.from_csr_values(brow, bcol, plan.assemble(M_local, 3))
+    A = K if not shift else _ops.Bsr3(brow, bcol, K.bval + float(shift) * M.bval)
+    H = amg.AmgHierarchy(A, _dof_mask(N, 3, fixed, dev), coords, K=K, M=M)
+    lam, S, info = modes.lobpcg(multigrid.MultilevelBackend(H), num_eigs, tol=tol, max_iter=max_iter)
+    d = H.describe()
+    info["levels"], info["operator_complexity"], info["setup_ms"], info["shift"] = d["levels"], d["operator_complexity"], d["setup_ms"], float(shift)
+    if verbose:
+        if info["status"] == "converged":
+            print(f"AMG LOBPCG converged after {info['iterations']} iterations on {3 * N} dofs ({len(H.L)} levels).")
+        else:
+            print(f"AMG LOBPCG did not converge within {max_iter} iterations; max residual {info['residuals'].max():.3e}.")
+    lam = torch.from_numpy(lam).to(device=dev, dtype=dtype)
+    modes_out = S[:, :num_eigs].contiguous().to(dtype)
+    return (lam, modes_out, info) if return_info else (lam, modes_out)
+
+
+def amg_buckling_modes(coords, elements, F, fixed, E, nu, num_eigs=4, tol=1e-8, max_iter=500, static_tol=1e-10, static_max_iter=500,
+                       integral_point=None, device="cuda:0", dtype=torch.float64, return_info=False, verbose=True):
+    """Linear buckling of a C3D4 or C3D10 mesh (not in the reference): what buckling_modes computes, with the Jacobi preconditioner
+    replaced by one V-cycle of smoothed-aggregation algebraic multigrid (femb200/amg.py, built from K and the coordinates) in both
+    the reference solve (PCG, buckling.static_multigrid) and LOBPCG.  Arguments, refusals and returns as buckling_modes; info also
+    holds `levels`, `operator_complexity` and `setup_ms` of the hierarchy."""
+    from femb200 import amg, buckling
+    dev = _ops.cuda_device(device)
+    elements = _ops.index(elements, dev)
+    if elements.dim() != 2 or elements.shape[1] not in (4, 10):
+        raise ValueError(f"elements must be [M,4] (C3D4) or [M,10] (C3D10), got {tuple(elements.shape)}")
+    _buckling_args(num_eigs, fixed)
+    coords = _ops.real(coords, dev, torch.float64)
+    N = coords.shape[0]
+    mask = _dof_mask(N, 3, fixed, dev)
+    plan = _ops.CsrPlan(elements, N, dev)
+    brow, bcol = plan.pattern(1)
+    if elements.shape[1] == 4:
+        Ke = _el.compute_c3d4_K_matrix(coords, elements, E, nu, device=dev, dtype=torch.float64)
+    else:
+        rule = torch.tensor(_el._exact_pts(_ops.C3D10, integral_point, torch.float64), dtype=torch.float64)
+        Ke = _el.compute_c3d10_K_matrix(coords, elements, E, nu, integral_point=rule, device=dev, dtype=torch.float64)
+    K = _ops.Bsr3.from_csr_values(brow, bcol, plan.assemble(Ke, 3))
+    del Ke
+    H = amg.AmgHierarchy(K, mask, coords, K=K)
+    u, static_its, static_res = buckling.static_multigrid(H, F, static_tol, static_max_iter)
+    u = u.reshape(N, 3)
+    if elements.shape[1] == 4:
+        KGe = _el.compute_c3d4_KG_matrix(coords, elements, u, E, nu, device=dev, dtype=torch.float64)
+    else:
+        KGe = _el.compute_c3d10_KG_matrix(coords, elements, u, E, nu, integral_point=rule, device=dev, dtype=torch.float64)
+    KG = _ops.Bsr3.from_csr_values(brow, bcol, plan.assemble(KGe, 3))
+    del KGe
+    lam, modes_out, info = buckling.solve(buckling.MultilevelBackend(H, KG), num_eigs, tol, max_iter)
+    d = H.describe()
+    info["static_iterations"], info["static_residual"] = static_its, static_res
+    info["levels"], info["operator_complexity"], info["setup_ms"] = d["levels"], d["operator_complexity"], d["setup_ms"]
+    if verbose:
+        _buckling_report("AMG", info, max_iter)
+    out = (torch.from_numpy(lam).to(device=dev, dtype=dtype), modes_out.contiguous().to(dtype), u.to(dtype))
+    return out + (info,) if return_info else out
+
+
 def static_structure_solver(coords, force, fixed, c3d4=None, c3d6=None, c3d8=None, s3=None, s4=None, material=None, u_init=None,
                             tol=1e-10, max_iter=1000, device="cuda:0", dtype=torch.float64, eps=1e-30, return_info=False, verbose=True):
     """Mixed-element static solve on [N,6] (solver.py:11-135): solids act on the translations, shells on all six dofs

@@ -341,6 +341,39 @@ int femb_mg_transfer(int64_t n_out, int64_t n_in, int64_t nnz, const int32_t* cr
                      const uint8_t* mask_out, int m, const double* X, int64_t ldx, int accumulate, double* Y, int64_t ldy,
                      femb_stream stream);
 
+/* Smoothed-aggregation multigrid (femb200/amg.py): every level is a square 3x3 block-CSR operator, the transfers are rectangular
+ * 3x3 block-CSR matrices (brow [rows+1], bcol int32, bval fp64 [nnzb, 3, 3]).  Aggregate a of the fine nodes gives the coarse
+ * pseudo-nodes 2a (translation columns) and 2a+1 (rotation columns).  Results do not depend on thread scheduling.
+ *   femb_mg_transfer_bsr3: Y[3i+d, j] (+)= mask_out[3i+d] (T X)[3i+d, j] for T with n_out block rows and block columns < n_in;
+ *     layout and rules as femb_mg_transfer.
+ *   femb_amg_aggregate: agg[nb] (int32) and *n_agg_host from the node graph (brow, bcol: a square block pattern); a node whose
+ *     three dofs are masked (mask NULL: none) gets -1.  Distance-2 maximal independent set by synchronous rounds (priority: a
+ *     fixed hash of the node id), roots take their neighbours, the rest join the neighbouring aggregate with the lowest id.
+ *   femb_amg_tentative: the tentative prolongator of `agg` (n_agg aggregates): prow [nb+1] (two blocks per aggregated node),
+ *     pcol / pval [2 n_aggregated], the coarse near-nullspace Bc [6 n_agg, 6] (global rigid-body modes), the coarse mask
+ *     mask_c [6 n_agg] and the coarse node coordinates coords_c [2 n_agg, 3] (both pseudo-nodes at the aggregate's centroid).
+ *     coords [nb, 3] are always given; the near-nullspace is the rigid-body modes of coords on the finest level (B NULL) and
+ *     B [3 nb, 6] on coarser ones; masked rows are zero.  Per aggregate the rotation columns are re-centred on its centroid and
+ *     scaled by 1 / its diameter, then CholQR2; a Cholesky pivot <= drop * (largest Gram diagonal) drops its column and masks its
+ *     coarse dof.
+ *   femb_bsr3_spgemm: C = X Y, X with n_rows block rows.  Call it twice: with ccol = cval = NULL it writes crow [n_rows+1] and
+ *     *nnz_host; then with ccol [nnz], cval [nnz, 3, 3] (and xval, yval) it writes the sorted columns and the values.  A row of
+ *     C may hold at most 2048 blocks: a wider row returns FEMB_ERR_UNSUPPORTED.
+ *   femb_bsr3_transpose: R = P^T (rrow [n_cols+1], rcol / rval [nnzb]), blocks transposed, each row of R in increasing column. */
+int femb_mg_transfer_bsr3(int64_t n_out, int64_t n_in, int64_t nnzb, const int32_t* trow, const int32_t* tcol, const double* tval,
+                          const uint8_t* mask_out, int m, const double* X, int64_t ldx, int accumulate, double* Y, int64_t ldy,
+                          femb_stream stream);
+int femb_amg_aggregate(int64_t nb, const int32_t* brow, const int32_t* bcol, const uint8_t* mask, int32_t* agg, int64_t* n_agg_host,
+                       femb_stream stream);
+int femb_amg_tentative(int64_t nb, int64_t n_agg, const int32_t* agg, const uint8_t* mask, const double* coords, const double* B,
+                       double drop, int32_t* prow, int32_t* pcol, double* pval, double* Bc, uint8_t* mask_c, double* coords_c,
+                       femb_stream stream);
+int femb_bsr3_spgemm(int64_t n_rows, const int32_t* xrow, const int32_t* xcol, const double* xval, const int32_t* yrow,
+                     const int32_t* ycol, const double* yval, int32_t* crow, int32_t* ccol, double* cval, int64_t* nnz_host,
+                     femb_stream stream);
+int femb_bsr3_transpose(int64_t n_rows, int64_t n_cols, int64_t nnzb, const int32_t* prow, const int32_t* pcol, const double* pval,
+                        int32_t* rrow, int32_t* rcol, double* rval, femb_stream stream);
+
 /* Jacobi diagonal of a CSR matrix: minv[i] = mask[i] ? 1/A_ii : 0 (the documented replacement for the
  * reference's broken compute_diagonal_preconditioner solver.py:814-833) */
 int femb_csr_jacobi(int64_t n, const int32_t* crow, const int32_t* col, const double* val, const uint8_t* mask,
